@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- throughput of the Forgex matching hot path on B200 (contract: see the task statement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2] [--lines L] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2] [--lines L] [--impl reference] [--dump-outputs DIR]
 
 Headline workload = BASELINE.json configs[1] ("c2"): `foo(bar|baz)` .in. over 100 M random ASCII lines of
 64-256 bytes, one pattern against N strings (flat buffer + int64 offsets).  A step = one pass of the
@@ -65,6 +65,24 @@ def known_traffic(cfg, algo_bytes):
     except Exception:
         pass
     return None
+
+
+DUMP_MAX_ELEMS = 1 << 20     # per array; at most seven arrays of 8-byte elements keep a dump under 64 MB
+
+
+def dump_index(n):
+    """the elements of an n-element output that --dump-outputs keeps: all of them up to DUMP_MAX_ELEMS, else a fixed
+    seeded sample (sorted, distinct), so that two runs with the same arguments write the same elements"""
+    if n <= DUMP_MAX_ELEMS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ELEMS, replace=False))
+
+
+def dump_output(torch, d, name, t):
+    """device tensor t -> d/<name>.npy (the elements dump_index picks): int64 spans as float64, which holds them exactly,
+    everything else as float32"""
+    a = t.reshape(-1)[torch.from_numpy(dump_index(t.numel())).to(t.device)].cpu().numpy()
+    np.save(os.path.join(d, name + ".npy"), a.astype(np.float64 if a.dtype == np.int64 else np.float32))
 
 
 class ClockSampler:
@@ -442,6 +460,13 @@ def measure_config(cfg, args, env):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_step = float(t.item()) / args.steps
+    if args.dump_outputs and rank == 0:
+        # what the last timed step handed its caller (every step overwrites the same output tensors)
+        if cfg == "c3":
+            dump_output(torch, args.dump_outputs, "c3_from", w["out"])
+            dump_output(torch, args.dump_outputs, "c3_to", w["out2"])
+        else:
+            dump_output(torch, args.dump_outputs, cfg + "_span" if cfg == "c4" else cfg, w["out"])
 
     split = cfg == "c4" and world > 1
     # match counts: the only cross-GPU exchange of a sharded batch (8 bytes per rank), outside the timed region
@@ -478,6 +503,8 @@ def measure_config(cfg, args, env):
         if world > 1:
             dist.all_reduce(gt, op=dist.ReduceOp.MAX)
         gms = float(gt.item()) / args.steps
+        if args.dump_outputs and rank == 0:
+            dump_output(torch, args.dump_outputs, "c2_general", gout)
         general = {"pattern": "\\w+@\\w+", "op": ".in.", "ms_per_step": gms, "value": w["text_bytes"] * world / (gms / 1000.0) / 1e9, "unit": "GB/s",
                    "sparse_used": gp.info()["sparse_used"], "matches_rank0": int(gout.sum(dtype=torch.int64).item())}
         if rank == 0 and world == 1 and not args.no_cpu:
@@ -645,7 +672,17 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-pin", action="store_true", help="do not bind the rank to its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step of each measured config computed (rank 0) as DIR/<name>.npy, "
+                         "float32 (float64 for int64 spans); outputs longer than %d elements as a fixed seeded sample"
+                         % DUMP_MAX_ELEMS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl == "reference":
+            ap.error("--dump-outputs records the GPU path's outputs; the reference arm runs other inputs")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     if args.warmup < 3 and args.impl == "b200" and not os.environ.get("FX_BENCH_ALLOW_SHORT_WARMUP"):
         args.warmup = 3
     if args.impl == "reference":
