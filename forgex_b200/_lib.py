@@ -13,6 +13,8 @@ FX_OP_MATCH, FX_OP_IN, FX_OP_REGEX = 0, 1, 2
 FX_TABLE_AUTO, FX_TABLE_SMEM, FX_TABLE_GLOBAL = 0, 1, 2
 FX_ERR_TREE_NODE_LIMIT, FX_ERR_DFA_STATE_CAP, FX_ERR_PREFILTER_UNSUPPORTED = 101, 102, 103
 FX_ERR_BAD_ARGUMENT, FX_ERR_NO_DEVICE, FX_ERR_WORK_BUDGET = 104, 105, 106
+FX_STATEMAP_MAP_WORDS, FX_STATEMAP_UNKNOWN = 98, -2
+FX_STATEMAP_WALK_WORDS, FX_STATEMAP_WALK_NEW, FX_STATEMAP_WALK_DONE = 4, -1, -2
 
 # every symbol include/forgex_b200.h declares (tests check that the library exports them all)
 SYMBOLS = [
@@ -20,6 +22,7 @@ SYMBOLS = [
     "fx_pattern_literals", "fx_pattern_tables", "fx_pattern_span_tables", "fx_pattern_nfa_tables", "fx_is_valid_regex", "fx_is_valid_regex_batch",
     "fx_match_fixed_dev", "fx_in_fixed_dev", "fx_match_batch_dev", "fx_in_batch_dev", "fx_regex_batch_dev",
     "fx_regex_buffer_work_bytes", "fx_regex_buffer_dev", "fx_buffer_scan_dev", "fx_buffer_scan_all_dev", "fx_buffer_finish_dev",
+    "fx_statemap_window_dev", "fx_statemap_combine", "fx_statemap_back_dev",
     "fx_match_fixed", "fx_in_fixed", "fx_match_batch", "fx_in_batch", "fx_regex_batch", "fx_regex_buffer",
     "fx_regex_count_batch_dev", "fx_regex_buffer_all_dev", "fx_regex_count_batch", "fx_regex_buffer_all",
     "fx_in", "fx_match", "fx_regex", "fx_in_value", "fx_match_value", "fx_regex_sub", "fx_launch_count",
@@ -81,6 +84,9 @@ def lib():
     L.fx_buffer_scan_dev.argtypes = [vp, u8p, i64, i64, i64, i64, C.c_int, C.c_int, vp, vp]
     L.fx_buffer_scan_all_dev.argtypes = [vp, u8p, i64, i64, i64, i64, C.c_int, C.c_int, vp, vp]
     L.fx_buffer_finish_dev.argtypes = [vp, u8p, i64, i64, C.c_int, vp, vp, vp]
+    L.fx_statemap_window_dev.argtypes = [vp, u8p, i64, i64, i64, i64, vp, vp, vp]
+    L.fx_statemap_combine.argtypes = [vp, vp, i64, i64, vp]
+    L.fx_statemap_back_dev.argtypes = [vp, u8p, i64, i64, i64, vp, vp]
     for name in ("fx_match_fixed", "fx_in_fixed"):
         getattr(L, name).argtypes = [vp, u8p, i64, i64, u8p]
     for name in ("fx_match_batch", "fx_in_batch"):

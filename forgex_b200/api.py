@@ -324,6 +324,27 @@ class Pattern:
         _check(L.lib().fx_buffer_finish_dev(self.h, _ptr(d_window), window_len, origin, int(is_last), _ptr(d_key),
                                             _ptr(d_from_to), self._stream()), "fx_buffer_finish_dev")
 
+    # ---- linear-time window form (include/forgex_b200.h: fx_statemap_*) ----
+    def statemap_window_dev(self, d_window, window_len, slab_lo, slab_hi, origin, d_map, d_work):
+        """slab map of window bytes [slab_lo, slab_hi) into d_map (FX_STATEMAP_MAP_WORDS int64)"""
+        assert d_map.numel() >= L.FX_STATEMAP_MAP_WORDS, "d_map is too small"
+        assert d_work.numel() * d_work.element_size() >= self.buffer_work_bytes(slab_hi - slab_lo), "d_work is too small"
+        _check(L.lib().fx_statemap_window_dev(self.h, _ptr(d_window), window_len, slab_lo, slab_hi, origin, _ptr(d_map),
+                                              _ptr(d_work), self._stream()), "fx_statemap_window_dev")
+
+    def statemap_combine(self, maps, text_len):
+        """slab maps (nmaps x FX_STATEMAP_MAP_WORDS, text order) -> int64[2] = (end of the match, declined); host-only"""
+        maps = np.ascontiguousarray(maps, dtype=np.int64).reshape(-1, L.FX_STATEMAP_MAP_WORDS)
+        out = np.zeros(2, dtype=np.int64)
+        _check(L.lib().fx_statemap_combine(self.h, _ptr(maps), maps.shape[0], text_len, _ptr(out)), "fx_statemap_combine")
+        return out
+
+    def statemap_back_dev(self, d_window, window_len, origin, text_len, d_walk):
+        """advance the backward walk d_walk (FX_STATEMAP_WALK_WORDS int64) over this window"""
+        assert d_walk.numel() >= L.FX_STATEMAP_WALK_WORDS, "d_walk is too small"
+        _check(L.lib().fx_statemap_back_dev(self.h, _ptr(d_window), window_len, origin, text_len, _ptr(d_walk),
+                                            self._stream()), "fx_statemap_back_dev")
+
 
 # ---- the reference's public API: one pattern, one text, compiled per call -----------------------
 def is_valid_regex(pattern):

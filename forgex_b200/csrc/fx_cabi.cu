@@ -1101,8 +1101,8 @@ inline size_t buffer_work_bytes(int64_t len) { return WORK_HEAD + (size_t)statem
 
 template <int FK>
 int launch_statemap_t(fx_pattern* p, const SpanParams& sp, StateMapParams mp, int fwd_bytes, const uint8_t* buf, int64_t len,
-                      cudaStream_t s, const unsigned long long* run_if) {
-    auto kern = k_statemap_regions<FK>;
+                      cudaStream_t s, const unsigned long long* run_if, bool window) {
+    auto kern = window ? k_statemap_regions<FK, true> : k_statemap_regions<FK, false>;
     const size_t smem = (size_t)((256 + fwd_bytes + 15) & ~15) + 256 * (1 + SM_M) * 2 + 256 + SM_WARPS * 32 * sizeof(SubMap) + SM_WARPS * 32 * 2 + 64;
     int bps = 0;
     int rc = occupancy_grid(kern, SM_WARPS * 32, smem, p->dev.sm_count, bps);
@@ -1123,17 +1123,17 @@ int launch_statemap_t(fx_pattern* p, const SpanParams& sp, StateMapParams mp, in
     g_launches++;
     rc = cuda_status(cudaGetLastError());
     if (rc) return rc;
-    k_statemap_compose<<<1, 1024, 0, s>>>(sp, mp, len, run_if);
+    if (window) k_statemap_compose<true><<<1, 1024, 0, s>>>(sp, mp, len, run_if);
+    else k_statemap_compose<false><<<1, 1024, 0, s>>>(sp, mp, len, run_if);
     g_launches++;
     return cuda_status(cudaGetLastError());
 }
 
-// the state-map scan + its finish, gated on *run_if != 0 (nullptr: always)
-int launch_statemap(fx_pattern* p, const uint8_t* buf, int64_t len, int64_t* from_to, unsigned long long* work, cudaStream_t s,
-                    const unsigned long long* run_if) {
+// the region and compose kernels of the state-map scan over buf[0, len), region maps in `work`.  back / pos0: see
+// StateMapParams (0 / 0 for a whole text); `result`: 2 words, or the slab map of the window form (window = true)
+int launch_statemap_scan(fx_pattern* p, const SpanParams& sp, const uint8_t* buf, int64_t len, int64_t back, int64_t pos0,
+                         unsigned long long* work, long long* result, cudaStream_t s, const unsigned long long* run_if, bool window) {
     const fx::ByteTable& st = p->prog.span_bt;
-    SpanParams sp;
-    fill_span_params(p, sp);
     StateMapParams mp;
     mp.reach = p->dev.sm_reach; mp.img = p->dev.sm_img; mp.sync = p->dev.sm_sync; mp.nreach = (int)p->sm_reach.size();
     uint8_t* maps = reinterpret_cast<uint8_t*>(work) + WORK_HEAD;
@@ -1141,20 +1141,30 @@ int launch_statemap(fx_pattern* p, const uint8_t* buf, int64_t len, int64_t* fro
     mp.rc = reinterpret_cast<uint16_t*>(maps);
     mp.re = mp.rc + cap * 32;
     mp.rl = reinterpret_cast<long long*>(maps + (size_t)cap * 32 * 4);
-    mp.result = reinterpret_cast<long long*>(work + 6);
+    mp.result = result;
     mp.region_bytes = 0; mp.nregions = 0;
+    mp.back = back; mp.pos0 = pos0;
     const int classed_bytes = (int)st.table.size() * 2;
     int fk = p->residency == FX_TABLE_GLOBAL ? 2 : p->dev.sp_direct ? 0 : classed_bytes <= SPAN_CLASSED_SMEM_BYTES ? 1 : 2;
     fk = env_int("FX_SPAN_FK", fk);
     if (fk == 0 && !p->dev.sp_direct) fk = 1;
     const int fwd_bytes = fk == 0 ? st.nstates * SPAN_ROW * 2 : fk == 1 ? classed_bytes : 0;
-    int rc = fk == 0 ? launch_statemap_t<0>(p, sp, mp, fwd_bytes, buf, len, s, run_if)
-           : fk == 1 ? launch_statemap_t<1>(p, sp, mp, fwd_bytes, buf, len, s, run_if)
-                     : launch_statemap_t<2>(p, sp, mp, fwd_bytes, buf, len, s, run_if);
+    return fk == 0 ? launch_statemap_t<0>(p, sp, mp, fwd_bytes, buf, len, s, run_if, window)
+         : fk == 1 ? launch_statemap_t<1>(p, sp, mp, fwd_bytes, buf, len, s, run_if, window)
+                   : launch_statemap_t<2>(p, sp, mp, fwd_bytes, buf, len, s, run_if, window);
+}
+
+// the state-map scan + its finish, gated on *run_if != 0 (nullptr: always)
+int launch_statemap(fx_pattern* p, const uint8_t* buf, int64_t len, int64_t* from_to, unsigned long long* work, cudaStream_t s,
+                    const unsigned long long* run_if) {
+    SpanParams sp;
+    fill_span_params(p, sp);
+    long long* result = reinterpret_cast<long long*>(work + 6);
+    int rc = launch_statemap_scan(p, sp, buf, len, 0, 0, work, result, s, run_if, false);
     if (rc) return rc;
     // with a prefix literal the answer only stands if the winner begins with the literal's own bytes (see launch_buffer)
     const bool check = p->prog.prefix_active && !p->prog.literal_only;
-    k_buffer_finish_span<<<1, 1, 0, s>>>(sp, buf, len, mp.result, from_to, work + 8, work + 9, run_if,
+    k_buffer_finish_span<<<1, 1, 0, s>>>(sp, buf, len, result, from_to, work + 8, work + 9, run_if,
                                          check ? p->dev.lits + p->prog.lit.all.size() : nullptr, check ? (int)p->prog.lit.prefix.size() : 0);
     g_launches++;
     return cuda_status(cudaGetLastError());
@@ -1654,6 +1664,81 @@ int fx_buffer_finish_dev(fx_pattern* p, const uint8_t* d_window, int64_t window_
     if (!d_key || !d_from_to) return FX_ERR_BAD_ARGUMENT;
     ScanWindow W{window_len, 0, window_len, origin, origin == 0 ? 1 : 0, is_last ? 1 : 0};
     return launch_finish(p, d_window, W, reinterpret_cast<const unsigned long long*>(d_key), d_from_to, 0, (cudaStream_t)stream);
+}
+
+// ---- linear-time window form: slab maps of the state-map scan, their combine, the backward walk across windows ----
+static_assert(FX_STATEMAP_MAP_WORDS == 2 + 3 * 32 && FX_STATEMAP_UNKNOWN == SM_MAP_UNKNOWN, "slab map layout");
+static_assert(FX_STATEMAP_WALK_NEW == SM_WALK_NEW && FX_STATEMAP_WALK_DONE == SM_WALK_DONE, "walk layout");
+
+// which patterns the window form serves (host-only: no device needed)
+static int statemap_window_served(const fx_pattern* p) {
+    if (!p) return FX_ERR_BAD_ARGUMENT;
+    if (p->prog.status != fx::OK) return p->prog.status;
+    if (p->prog.op != FX_OP_REGEX) return FX_ERR_BAD_ARGUMENT;
+    if (p->prog.nfa_engine) return FX_ERR_DFA_STATE_CAP;
+    // a prefix literal restricts Forgex's candidates to its occurrences, which may lie in another slab
+    if (p->prog.literal_only || p->prog.prefix_active) return FX_ERR_PREFILTER_UNSUPPORTED;
+    if (!p->statemap) return FX_ERR_DFA_STATE_CAP;
+    return FX_OK;
+}
+
+int fx_statemap_window_dev(fx_pattern* p, const uint8_t* d_window, int64_t window_len, int64_t slab_lo, int64_t slab_hi,
+                           int64_t origin, int64_t* d_map, void* d_work, void* stream) {
+    int rc = check_ready(p, FX_OP_REGEX);
+    if (rc) return rc;
+    if ((rc = statemap_window_served(p))) return rc;
+    if (!d_map || !d_work || (!d_window && window_len > 0) || origin < 0 || slab_lo < 0 || slab_lo > slab_hi ||
+        slab_hi > window_len)
+        return FX_ERR_BAD_ARGUMENT;
+    const int64_t back = origin + slab_lo < SM_LOOKBACK ? origin + slab_lo : SM_LOOKBACK;
+    if (slab_lo < back) return FX_ERR_BAD_ARGUMENT;          // the look-back in front of the slab is missing
+    SpanParams sp;
+    fill_span_params(p, sp);
+    return launch_statemap_scan(p, sp, d_window + slab_lo, slab_hi - slab_lo, back, origin + slab_lo,
+                                static_cast<unsigned long long*>(d_work), reinterpret_cast<long long*>(d_map),
+                                (cudaStream_t)stream, nullptr, true);
+}
+
+int fx_statemap_combine(const fx_pattern* p, const int64_t* maps, int64_t nmaps, int64_t text_len, int64_t out[2]) {
+    int rc = statemap_window_served(p);
+    if (rc) return rc;
+    if (!out || nmaps < 0 || (nmaps > 0 && !maps) || text_len < 0) return FX_ERR_BAD_ARGUMENT;
+    const fx::ByteTable& st = p->prog.span_bt;
+    int64_t s = st.start;
+    int64_t last = (st.flags[(size_t)st.start] & fxk::SF_ACC) ? 0 : -1;
+    out[0] = -1; out[1] = 0;
+    for (int64_t i = 0; i < nmaps && s != 0; i++) {
+        const int64_t* m = maps + i * FX_STATEMAP_MAP_WORDS;
+        if (m[0] == 2) continue;                             // empty slab: the identity
+        if (m[0] != 0 || m[1] < 0 || m[1] > 32) { out[1] = 1; return FX_OK; }
+        int hit = -1;
+        for (int k = 0; k < (int)m[1]; k++) if (m[2 + k] == s) hit = k;
+        if (hit < 0 || m[66 + hit] == FX_STATEMAP_UNKNOWN) { out[1] = 1; return FX_OK; }
+        s = m[34 + hit];
+        if (s < 0 || s >= st.nstates) return FX_ERR_BAD_ARGUMENT;
+        if (m[66 + hit] >= 0) last = m[66 + hit];
+    }
+    if (s != 0) {                                            // end of the text: pending bytes replay, the trailing NUL is consumed
+        const uint32_t e = st.endinfo[(size_t)s];
+        if (e & 3u) last = text_len + 1 - (int64_t)(e & 3u);
+        if (e & 4u) last = text_len + 1;
+    }
+    out[0] = last;
+    return FX_OK;
+}
+
+int fx_statemap_back_dev(fx_pattern* p, const uint8_t* d_window, int64_t window_len, int64_t origin, int64_t text_len,
+                         int64_t* d_walk, void* stream) {
+    int rc = check_ready(p, FX_OP_REGEX);
+    if (rc) return rc;
+    if ((rc = statemap_window_served(p))) return rc;
+    if (!d_walk || (!d_window && window_len > 0) || window_len < 0 || origin < 0 || origin + window_len > text_len)
+        return FX_ERR_BAD_ARGUMENT;
+    SpanParams sp;
+    fill_span_params(p, sp);
+    k_statemap_back<<<1, 1, 0, (cudaStream_t)stream>>>(sp, d_window, origin, window_len, text_len, reinterpret_cast<long long*>(d_walk));
+    g_launches++;
+    return cuda_status(cudaGetLastError());
 }
 
 // ---- all matches / match counts (the loop a caller of regex() writes: match, then regex() again on text(to+1:)) ----

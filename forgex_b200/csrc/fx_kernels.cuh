@@ -2787,8 +2787,15 @@ struct StateMapParams {
     uint16_t* rc;               // nregions x 32: region candidates (0xFFFF = unused lane; all 0xFFFF = the region declined)
     uint16_t* re;               // nregions x 32: end state per candidate
     long long* rl;              // nregions x 32: last accept (text position, -1 none) per candidate
-    long long* result;          // [0] = last accept of the whole text (-1 none), [1] = status (0 ok, 1 declined)
+    long long* result;          // [0] = last accept of the whole text (-1 none), [1] = status (0 ok, 1 declined);
+                                // window form: the slab map (FX_STATEMAP_MAP_WORDS words, see k_statemap_compose)
+    int64_t back;               // bytes of the text in front of buf[0] that the first region may read (<= SM_LOOKBACK);
+                                // 0: buf begins the text, and the walk starts in the automaton's start state
+    int64_t pos0;               // text position of buf[0]: added to every last accept, so slab maps speak whole-text positions
 };
+static constexpr long long SM_NO_ACCEPT = -(1ll << 62);     // "no accept yet": in a slab an accept may lie up to 2 bytes
+                                                            // in front of buf (a replay across the cut), so -1 is a position
+static constexpr long long SM_MAP_UNKNOWN = -2;             // slab map: this key met a region that does not know it
 
 // one forward step on 64-bit positions
 #define FX_SM_STEP(T, st, last, b, jj)                                            \
@@ -2812,11 +2819,14 @@ struct SubMap {
     uint8_t pad;
 };
 
-template <int FK>
+// WINDOW: buf is a slab that may not begin the text (mp.back, mp.pos0); the whole-text form compiles without them
+template <int FK, bool WINDOW>
 __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParams sp, StateMapParams mp,
                                                                       const uint8_t* __restrict__ buf, int64_t len, int fwd_bytes,
                                                                       const unsigned long long* __restrict__ run_if) {
     if (run_if != nullptr && *run_if == 0) return;            // the budgeted candidate scan has answered
+    const int64_t back = WINDOW ? mp.back : 0;
+    constexpr long long NO_ACC = WINDOW ? SM_NO_ACCEPT : -1;   // "no accept yet"
     extern __shared__ __align__(128) uint8_t smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t FULL = 0xffffffffu;
@@ -2889,11 +2899,11 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
         int cnt = 0;
         bool wide = false;
         __syncwarp();
-        if (r0 == 0) {
+        if (r0 == 0 && back == 0) {
             if (lane == 0) s_rc[0] = (uint16_t)sp.start;
             cnt = 1;
         } else {
-            const int64_t w0 = r0 > SM_LOOKBACK ? r0 - SM_LOOKBACK : 0;
+            const int64_t w0 = r0 - SM_LOOKBACK > -back ? r0 - SM_LOOKBACK : -back;
             for (int k = 0; k < mp.nreach && !wide; k += 32) {
                 uint32_t st = k + lane < mp.nreach ? (uint32_t)__ldg(mp.reach + k + lane) : 0u;
                 for (int64_t j = w0; j < r0; j++) st = T.next(st, (uint32_t)__ldg(buf + j)) & W_SSTATE;
@@ -2914,7 +2924,7 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
         }
         const uint32_t mycand = lane < cnt ? (uint32_t)s_rc[lane] : 0u;
         uint32_t c = mycand;                                 // this lane's chain state
-        long long L = -1;                                    // its last accept
+        long long L = NO_ACC;                                // its last accept
         // ---- segments of 32 sub-chunks ----
         for (int64_t k0 = kr0; k0 < kr1; k0 += 32) {
             const int64_t kb = k0 + lane;
@@ -2933,7 +2943,7 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
                 uint32_t st[SM_M] = {0, 0, 0, 0};
                 int nc = 0;
                 bool unknown = false;
-                if (b == 0) { st[0] = (uint32_t)sp.start; nc = 1; }
+                if (b == 0 && back == 0) { st[0] = (uint32_t)sp.start; nc = 1; }
                 else {
                     const uint32_t c1 = __ldg(buf + b - 1);
                     const uint32_t n1 = s_img[c1 * (1 + SM_M)];
@@ -2941,7 +2951,7 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
                         nc = (int)n1;
 #pragma unroll
                         for (int k = 0; k < SM_M; k++) if (k < nc) st[k] = s_img[c1 * (1 + SM_M) + 1 + k];
-                    } else if (b >= 2) {
+                    } else if (b + back >= 2) {
                         const uint32_t c2 = __ldg(buf + b - 2);
                         const uint32_t n2 = s_img[c2 * (1 + SM_M)];
                         if (n2 <= SM_M) {
@@ -2971,7 +2981,7 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
                     uint32_t active = 0, root = 0x3210u;     // bit k: candidate k is walked; nibble k of root: whom k follows
 #pragma unroll
                     for (int k = 0; k < SM_M; k++) if (k < nc && st[k] != 0) active |= 1u << k;
-                    long long last = -1;
+                    long long last = NO_ACC;
                     int owner = -1;
                     bool complex = false;
                     int64_t j = b;
@@ -3030,7 +3040,7 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
                         // held an event is walked again with the books.
                         const int k1 = __ffs(active) - 1;
                         uint32_t cur = k1 == 0 ? st[0] : k1 == 1 ? st[1] : k1 == 2 ? st[2] : st[3];
-                        long long l2 = -1;
+                        long long l2 = NO_ACC;
                         // (whole aligned 16-byte blocks are loaded even where only part of one belongs to the sub-chunk:
                         //  a block that holds one byte of the text lies inside the text's allocation)
                         if ((gbuf + (uintptr_t)j) & 15) {                        // head: up to the next 16-byte boundary
@@ -3069,7 +3079,7 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
                             walk_block(v, 0, (int)(e - j), cur, l2, j);
                             j = e;
                         }
-                        if (l2 >= 0) { last = l2; owner = k1; }
+                        if (WINDOW ? l2 != NO_ACC : l2 >= 0) { last = l2; owner = k1; }
 #pragma unroll
                         for (int k = 0; k < SM_M; k++) if (k == k1) st[k] = cur;
                         if (cur == 0) active = 0;
@@ -3087,7 +3097,7 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
                             if ((int)r == owner) om |= 1u << k;
                         }
                         mine.owner_mask = (uint16_t)om;
-                        mine.last = last >= 0 ? (int32_t)(last - b) : INT32_MIN;
+                        mine.last = (WINDOW ? last != NO_ACC : last >= 0) ? (int32_t)(last - b) : INT32_MIN;
                     }
                 }
             }
@@ -3118,7 +3128,7 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
         }
         mp.rc[reg * 32 + lane] = lane < cnt ? (uint16_t)mycand : (uint16_t)0xFFFFu;
         mp.re[reg * 32 + lane] = (uint16_t)c;
-        mp.rl[reg * 32 + lane] = L;
+        mp.rl[reg * 32 + lane] = WINDOW ? (L == NO_ACC ? -1 : L + mp.pos0) : L;
     }
 }
 
@@ -3127,9 +3137,22 @@ __global__ void __launch_bounds__(SM_WARPS * 32, 2) k_statemap_regions(SpanParam
 // through the range (a lookup among a region's 32 keys is 32 shuffles; eight regions' maps are fetched at a time) --
 // and warp 0 then chains the 32 range maps from the automaton's start state.  (One warp walking the ~19 000 regions of
 // a multi-GiB text one after the other took 13 ms, 4.2 ms with batched loads; this form takes a few hundred us.)
+// WINDOW: buf is a slab of a text split across GPUs.  The true state at the slab's start is unknown here, so warp 0
+// chains the 32 range maps for EVERY key of region 0 (one per lane) and writes the slab map to mp.result:
+//   [0] status (0 ok, 1 declined, 2 empty slab), [1] key count, [2..33] keys, [34..65] end states,
+//   [66..97] last accepts in text positions (-1 none, SM_MAP_UNKNOWN: the key met a region that does not know it).
+// No end-of-text step: fx_statemap_combine applies it after the last slab.
+template <bool WINDOW>
 __global__ void __launch_bounds__(1024) k_statemap_compose(SpanParams sp, StateMapParams mp, int64_t len,
                                                            const unsigned long long* __restrict__ run_if) {
     if (run_if != nullptr && *run_if == 0) return;
+    if (WINDOW && len == 0) {
+        if (threadIdx.x < 32) {
+            mp.result[2 + threadIdx.x] = 0; mp.result[34 + threadIdx.x] = 0; mp.result[66 + threadIdx.x] = -1;
+            if (threadIdx.x == 0) { mp.result[0] = 2; mp.result[1] = 0; }
+        }
+        return;
+    }
     __shared__ uint16_t r_key[32][32], r_end[32][32];
     __shared__ long long r_l[32][32];
     __shared__ uint8_t r_bad[32][32];
@@ -3173,6 +3196,27 @@ __global__ void __launch_bounds__(1024) k_statemap_compose(SpanParams sp, StateM
     }
     __syncthreads();
     if (warp != 0) return;
+    if (WINDOW) {
+        const uint32_t key = r_key[0][lane];
+        const bool live = key != 0xFFFFu;
+        uint32_t cs = r_end[0][lane];
+        long long L = r_l[0][lane];
+        bool unknown = r_bad[0][lane] != 0;
+        for (int w = 1; w < 32 && live && cs != 0 && !unknown; w++) {
+            if ((int64_t)w * per >= n) break;
+            int src = -1;
+            for (int q = 0; q < 32; q++) if (r_key[w][q] == cs) src = q;
+            if (src < 0 || r_bad[w][src]) { unknown = true; break; }
+            cs = r_end[w][src];
+            if (r_l[w][src] >= 0) L = r_l[w][src];
+        }
+        const int nkeys = __popc(__ballot_sync(FULL, live));
+        if (lane == 0) { mp.result[0] = nkeys == 0 ? 1 : 0; mp.result[1] = nkeys; }   // no key: region 0 declined
+        mp.result[2 + lane] = live ? key : 0;
+        mp.result[34 + lane] = live && !unknown ? cs : 0;
+        mp.result[66 + lane] = !live ? -1 : unknown ? SM_MAP_UNKNOWN : L;
+        return;
+    }
     uint32_t st = (uint32_t)sp.start;
     long long L = sp.start_acc ? 0 : -1;
     int status = 0;
@@ -3195,15 +3239,16 @@ __global__ void __launch_bounds__(1024) k_statemap_compose(SpanParams sp, StateM
     if (lane == 0) { mp.result[0] = status == 0 ? L : -1; mp.result[1] = status; }
 }
 
-// backward half on 64-bit positions (one thread): the leftmost start of the match that ends at `last`
-__device__ inline long long span_backward64(const SpanParams& sp, const uint8_t* __restrict__ buf, long long len, long long last) {
+// The backward half on 64-bit positions (one thread), as a resumable step loop over (pos, reverse state r, best so far).
+// Text byte p is win[p - org].  The loop steps while r lives and pos > 0, and -- unless the window begins the text
+// (org == 0) -- only while the next character's decode stays inside the window (pos - 4 >= org): a walk stopped there
+// is continued by whoever holds the bytes in front.
+__device__ inline void span_back_steps(const SpanParams& sp, const uint8_t* __restrict__ win, long long org, long long& pos,
+                                       uint32_t& r, long long& best) {
     SpanRev<false> R;
     R.s_delta = R.s_page = R.s_mixed = 0;
-    uint32_t r = (uint32_t)sp.rstart;
-    long long pos = last;
-    if (last > len) { r = R.delta(sp, r, (uint32_t)sp.nul_class) & 0x7FFFu; pos = len; }
-    long long best = -2;
-    while (r != 0 && pos > 0) {
+    const uint8_t* buf = win - org;          // (only ever dereferenced at positions >= org)
+    while (r != 0 && pos > 0 && (org == 0 || pos - 4 >= org)) {
         uint32_t c = __ldg(buf + pos - 1);
         long long q = pos - 1;
         uint32_t cp = c;
@@ -3231,12 +3276,63 @@ __device__ inline long long span_backward64(const SpanParams& sp, const uint8_t*
         pos = q;
         if (w & 0x8000u) best = pos;
     }
+}
+
+// start of the backward walk from the end `last` of the match (the trailing NUL first when it was consumed)
+__device__ inline void span_back_begin(const SpanParams& sp, long long len, long long last, long long& pos, uint32_t& r,
+                                       long long& best) {
+    SpanRev<false> R;
+    R.s_delta = R.s_page = R.s_mixed = 0;
+    r = (uint32_t)sp.rstart;
+    pos = last;
+    if (last > len) { r = R.delta(sp, r, (uint32_t)sp.nul_class) & 0x7FFFu; pos = len; }
+    best = -2;
+}
+
+// end of the backward walk (it stopped, or reached position 0): the leading NUL's step, then `from` (0: none)
+__device__ inline long long span_back_end(const SpanParams& sp, long long pos, uint32_t r, long long best) {
     if (r != 0 && pos == 0) {
+        SpanRev<false> R;
+        R.s_delta = R.s_page = R.s_mixed = 0;
         const uint32_t w = R.delta(sp, r, (uint32_t)sp.nul_class);
         if ((w & 0x7FFFu) != 0 && (w & 0x8000u)) best = -1;
     }
     if (best == -2) return 0;
     return best < 0 ? 1 : best + 1;
+}
+
+// the leftmost start of the match that ends at `last`, the whole text in buf
+__device__ inline long long span_backward64(const SpanParams& sp, const uint8_t* __restrict__ buf, long long len, long long last) {
+    long long pos, best;
+    uint32_t r;
+    span_back_begin(sp, len, last, pos, r, best);
+    span_back_steps(sp, buf, 0, pos, r, best);
+    return span_back_end(sp, pos, r, best);
+}
+
+// The backward walk of a text split across GPUs (one thread), over the window win[0, wlen) = text[org, org + wlen).
+// walk = {pos, best, reverse state, end}: the caller starts it as {0, 0, SM_WALK_NEW, end of the match}; each call
+// walks as far as the window allows.  When the walk is over: walk = {from, to, SM_WALK_DONE, end}, exactly
+// k_buffer_finish_span's answer for the whole text; otherwise it goes on at the holder of text byte pos - 1.
+static constexpr long long SM_WALK_NEW = -1, SM_WALK_DONE = -2;
+__global__ void k_statemap_back(SpanParams sp, const uint8_t* __restrict__ win, int64_t org, int64_t wlen, int64_t len,
+                                long long* __restrict__ walk) {
+    const long long state = walk[2], last = walk[3];
+    if (state == SM_WALK_DONE) return;
+    long long pos = walk[0], best = walk[1];
+    uint32_t r = (uint32_t)state;
+    if (state == SM_WALK_NEW) {
+        // the blank-text rule (api_internal_m.F90:68-74) and "no match"; a text of one byte lies in every window
+        const bool blank = len == 0 || (len == 1 && org == 0 && wlen >= 1 && __ldg(win) == 0x20);
+        if (blank || last <= 0) { walk[0] = 0; walk[1] = 0; walk[2] = SM_WALK_DONE; return; }
+        span_back_begin(sp, len, last, pos, r, best);
+    }
+    span_back_steps(sp, win, org, pos, r, best);
+    if (r != 0 && pos > 0) { walk[0] = pos; walk[1] = best; walk[2] = r; return; }     // at the window's front edge
+    const long long f = span_back_end(sp, pos, r, best);
+    walk[0] = f > 0 ? f : 0;
+    walk[1] = f > 0 ? (last < len ? last : len) : 0;
+    walk[2] = SM_WALK_DONE;
 }
 
 // finish of the state-map scan: (from, to) from the end position the compose step found.  `done`: set to 1 when this

@@ -10,12 +10,23 @@ search are independent attempts.  No text ever crosses GPUs.
             start of its slab; one all-reduce(MIN) of that 8-byte key; the owner of the winner computes the span;
             one broadcast of 16 bytes.
 
-Everything here is host logic over a `scan` / `finish` pair, so it runs unchanged on CPU with the gloo backend
-(tests/test_dist_gloo.py plugs a Python model of the kernels in) and on GPUs with NCCL (plugs the C ABI in).
+  buffer, linear time (statemap_search)
+            contiguous byte slabs plus 64 bytes of look-back, no halo; each rank computes the state map of its slab
+            (the chunked state-map scan of the single-GPU path, every state that can arrive at the slab as a key); one
+            all-gather of the maps; every rank combines them into the end of the match; a backward walk from that end
+            finds the start, handed to the rank in front by a 32-byte broadcast whenever it reaches its window's front
+            edge; the last broadcast carries the span.  No attempt is replayed, so no pattern makes it quadratic.
+
+Everything here is host logic over callbacks (`scan` / `finish`, `window_map` / `combine` / `back`), so it runs
+unchanged on CPU with the gloo backend (tests/test_dist_gloo.py and tests/test_statemap_windows.py plug Python models of
+the kernels in) and on GPUs with NCCL (plugs the C ABI in).
 """
 import numpy as np
 
 NO_START = (1 << 64) - 1
+STATEMAP_LOOKBACK = 64                 # bytes in front of a slab the slab map reads (SM_LOOKBACK of the kernels)
+STATEMAP_MAP_WORDS = 98                # FX_STATEMAP_MAP_WORDS: status, key count, 32 keys, 32 end states, 32 last accepts
+STATEMAP_WALK_NEW, STATEMAP_WALK_DONE = -1, -2
 
 
 def shard_strings(offsets, world, rank):
@@ -47,6 +58,11 @@ def window_for_slab(length, lo, hi, halo):
     w_lo = max(0, lo - 3)
     w_hi = min(length, hi + halo)
     return w_lo, w_hi
+
+
+def window_for_statemap_slab(length, lo, hi):
+    """the bytes a rank must hold for the linear-time form over [lo, hi): STATEMAP_LOOKBACK bytes of look-back, no halo"""
+    return max(0, lo - STATEMAP_LOOKBACK), hi
 
 
 def all_reduce_int(value, op, group=None, device=None):
@@ -147,6 +163,60 @@ def buffer_search(scan, finish, length, rank, world, slab, window=None, group=No
     return f, t, undecided_total
 
 
+def statemap_search(window_map, combine, back, length, rank, world, slab, group=None, device=None, stats=None):
+    """Leftmost-longest search of one pattern in one buffer split across ranks, in time linear in the text.
+
+    window_map(lo, hi) -> STATEMAP_MAP_WORDS integers: the slab map of this rank's slab [lo, hi) (fx_statemap_window_dev).
+    combine(maps) -> (end, declined): the slab maps of all ranks chained in text order (fx_statemap_combine).
+    back(walk) -> walk: the backward walk advanced over this rank's window (fx_statemap_back_dev); walk = [pos, best,
+        reverse state, end], started as [0, 0, STATEMAP_WALK_NEW, end], over when walk[2] == STATEMAP_WALK_DONE, and
+        then walk[:2] = (from, to).
+    Collectives per search: one all-gather of STATEMAP_MAP_WORDS + 2 integers, then one 32-byte broadcast per rank the
+    walk visits -- the first from the rank that holds byte end - 1 (the last rank when the trailing NUL was consumed),
+    one more per slab boundary the match crosses (stats["hops"]); the last one carries the span.  Nothing when there is
+    no match.  Returns (from, to, declined); every rank gets the same answer.  declined: more than 32 states can arrive
+    at some slab on the true path, (from, to) = (0, 0) is then no answer: search with buffer_search instead.
+    """
+    import torch
+    import torch.distributed as dist
+    lo, hi = slab
+    multi = dist.is_initialized() and world > 1
+    table = gather_ints(list(window_map(lo, hi)) + [lo, hi], group, device)
+    maps = [row[:STATEMAP_MAP_WORDS] for row in table]
+    slabs = [(row[STATEMAP_MAP_WORDS], row[STATEMAP_MAP_WORDS + 1]) for row in table]
+    end, declined = combine(maps)
+    hops = 0
+    if stats is not None:
+        stats["hops"] = 0
+    if declined:
+        return 0, 0, True
+    if end <= 0:
+        return 0, 0, False
+
+    def owner(b):
+        return next(r for r, (a, z) in enumerate(slabs) if a <= b < z)
+
+    walker = owner(end - 1) if end <= length else len(slabs) - 1
+    walk = torch.tensor([0, 0, STATEMAP_WALK_NEW, end], dtype=torch.int64, device=device)
+    while True:
+        if rank == walker:
+            walk.copy_(torch.tensor(back(walk.cpu().tolist()), dtype=torch.int64))
+        if multi:
+            dist.broadcast(walk, src=walker if group is None else dist.get_global_rank(group, walker), group=group)
+        pos, best, state, _ = walk.cpu().tolist()
+        if state == STATEMAP_WALK_DONE:
+            break
+        nxt = owner(pos - 1)
+        if nxt == walker:
+            raise RuntimeError("backward walk stopped at %d inside the window of rank %d: the window lacks its look-back"
+                               % (pos, walker))
+        walker = nxt
+        hops += 1
+    if stats is not None:
+        stats["hops"] = hops
+    return pos, best, False
+
+
 class _GpuWindow:
     """a rank's piece of the text on its GPU: slab + 3 bytes of look-back + a look-ahead halo that can grow"""
 
@@ -221,3 +291,53 @@ def gpu_buffer_search(pattern_obj, d_window, window_origin, length, rank, world,
 
     return buffer_search(scan, finish, length, rank, world, slab, None, group, dev, scan_all if prefixed else None,
                          widen=win.widen if world > 1 else None, stats=stats)
+
+
+def gpu_buffer_search_linear(pattern_obj, d_window, window_origin, length, rank, world, slab, group=None, stats=None):
+    """statemap_search over the C ABI: d_window is this rank's CUDA tensor holding text[window_for_statemap_slab(...)].
+
+    Patterns the linear-time form does not serve (a prefix literal, a literal-only pattern, no span path, the NFA
+    engine) and searches it declines are answered by gpu_buffer_search on the same window, whose look-ahead halo starts
+    empty and grows on demand (what that scan does not serve either -- a sequential candidate list, an NFA-engine
+    handle -- raises its ForgexError).  stats["route"] = "statemap" or "scan".  Returns (from, to)."""
+    import torch
+    from .api import ForgexError
+    from . import _lib
+    lo, hi = slab
+    assert (window_origin, window_origin + d_window.numel()) == window_for_statemap_slab(length, lo, hi), \
+        "the window must come from window_for_statemap_slab"
+    stats = {} if stats is None else stats
+    dev = d_window.device
+    try:
+        pattern_obj.statemap_combine(np.zeros((0, STATEMAP_MAP_WORDS), dtype=np.int64), length)     # (host-only)
+        served = True
+    except ForgexError as e:
+        if e.status not in (_lib.FX_ERR_DFA_STATE_CAP, _lib.FX_ERR_PREFILTER_UNSUPPORTED):
+            raise
+        served = False                  # a property of the pattern: every rank takes the same route
+    if served:
+        wlen = d_window.numel()
+        d_map = torch.empty(STATEMAP_MAP_WORDS, dtype=torch.int64, device=dev)
+        work = torch.empty(pattern_obj.buffer_work_bytes(hi - lo), dtype=torch.uint8, device=dev)
+        d_walk = torch.empty(4, dtype=torch.int64, device=dev)
+
+        def window_map(a, b):
+            pattern_obj.statemap_window_dev(d_window, wlen, a - window_origin, b - window_origin, window_origin, d_map, work)
+            return d_map.cpu().tolist()
+
+        def combine(maps):
+            out = pattern_obj.statemap_combine(np.array(maps, dtype=np.int64), length)
+            return int(out[0]), bool(out[1])
+
+        def back(walk):
+            d_walk.copy_(torch.tensor(walk, dtype=torch.int64))
+            pattern_obj.statemap_back_dev(d_window, wlen, window_origin, length, d_walk)
+            return d_walk.cpu().tolist()
+
+        f, t, declined = statemap_search(window_map, combine, back, length, rank, world, slab, group, dev, stats)
+        if not declined:
+            stats["route"] = "statemap"
+            return f, t
+    stats["route"] = "scan"
+    f, t, _ = gpu_buffer_search(pattern_obj, d_window, window_origin, length, rank, world, slab, group, stats)
+    return f, t

@@ -279,6 +279,30 @@ module forgex_b200_m
          integer(c_int), value :: is_last
          integer(c_int) :: status
       end function
+      ! linear-time window form (UNVERIFIED like the rest of this module): slab map per rank, the host combine of the
+      ! gathered maps (FX_STATEMAP_MAP_WORDS = 98 int64 per rank), the backward walk (FX_STATEMAP_WALK_WORDS = 4 int64)
+      function fx_statemap_window_dev(p, d_window, window_len, slab_lo, slab_hi, origin, d_map, d_work, stream) &
+            bind(c, name='fx_statemap_window_dev') result(status)
+         import :: c_ptr, c_int64_t, c_int
+         type(c_ptr), value :: p, d_window, d_map, d_work, stream
+         integer(c_int64_t), value :: window_len, slab_lo, slab_hi, origin
+         integer(c_int) :: status
+      end function
+      function fx_statemap_combine(p, maps, nmaps, text_len, out) bind(c, name='fx_statemap_combine') result(status)
+         import :: c_ptr, c_int64_t, c_int
+         type(c_ptr), value :: p
+         integer(c_int64_t), intent(in) :: maps(*)
+         integer(c_int64_t), value :: nmaps, text_len
+         integer(c_int64_t), intent(out) :: out(2)
+         integer(c_int) :: status
+      end function
+      function fx_statemap_back_dev(p, d_window, window_len, origin, text_len, d_walk, stream) &
+            bind(c, name='fx_statemap_back_dev') result(status)
+         import :: c_ptr, c_int64_t, c_int
+         type(c_ptr), value :: p, d_window, d_walk, stream
+         integer(c_int64_t), value :: window_len, origin, text_len
+         integer(c_int) :: status
+      end function
       ! ---- the Fortran-side compile route (forgex_b200_tables_m) ----
       function fx_compile_from_dfa(op, cuts, ncls, delta, nstates, accept, q0, all, all_len, prefix, prefix_len, &
                                    suffix, suffix_len, out) bind(c, name='fx_compile_from_dfa') result(status)
@@ -297,6 +321,7 @@ module forgex_b200_m
    public :: fx_match_fixed_dev, fx_in_fixed_dev, fx_match_batch_dev, fx_in_batch_dev, fx_regex_batch_dev, fx_regex_count_batch_dev
    public :: fx_regex_buffer_work_bytes, fx_regex_buffer_dev, fx_regex_buffer_all_dev
    public :: fx_buffer_scan_dev, fx_buffer_scan_all_dev, fx_buffer_finish_dev
+   public :: fx_statemap_window_dev, fx_statemap_combine, fx_statemap_back_dev
 
 contains
 

@@ -60,11 +60,15 @@ enum {
     FX_ERR_DFA_STATE_CAP = 102,        /* eager construction exceeds 16383 states (Forgex's own ceiling for the
                                           lazily visited states: src/lazy_dfa/lazy_dfa_graph_m.F90:90-92) AND the NFA
                                           engine cannot take over (more than 8191 NFA states), or an entry point that
-                                          needs the table engine was called on an NFA-engine handle */
+                                          needs the table engine was called on an NFA-engine handle; the linear-time
+                                          window form (fx_statemap_*) also answers it for a pattern without the span
+                                          path (fx_pattern_info.statemap == 0) */
     FX_ERR_PREFILTER_UNSUPPORTED = 103,/* WINDOW forms only (a text split across GPUs): the pattern's candidate list is
                                           sequential -- a prefix literal that can overlap itself, or a suffix literal
                                           (src/essential/utility_m.f90:58-117).  fx_regex_buffer* itself answers such
-                                          patterns (one thread replays the reference's rule: exact, slow) */
+                                          patterns (one thread replays the reference's rule: exact, slow).  The
+                                          linear-time window form (fx_statemap_*) answers it for every pattern with an
+                                          extracted prefix literal and for literal-only patterns */
     FX_ERR_BAD_ARGUMENT = 104,
     FX_ERR_NO_DEVICE = 105,
     FX_ERR_WORK_BUDGET = 106           /* fx_regex_buffer* only: Forgex's own loop would need more than 16 byte steps per text
@@ -223,6 +227,39 @@ int fx_buffer_scan_all_dev(fx_pattern* p, const uint8_t* d_window, int64_t windo
                            int64_t origin, int is_first, int is_last, uint64_t* d_best, void* stream);
 int fx_buffer_finish_dev(fx_pattern* p, const uint8_t* d_window, int64_t window_len, int64_t origin, int is_last,
                          const uint64_t* d_key, int64_t* d_from_to, void* stream);
+
+/* Linear-time window form: the chunked state-map scan of fx_regex_buffer* over a text split across GPUs.  Each GPU
+ * computes the SLAB MAP of its slab, the maps are gathered and combined (the same answer on every GPU), and a backward
+ * walk finds the start of the match, handed from GPU to GPU when the match crosses slabs.  No attempt is replayed:
+ * the work is linear in the text whatever the pattern, where the window scan above runs Forgex's own candidate loop.
+ * Served: FX_OP_REGEX handles with the span path (fx_pattern_info.statemap) and no prefix literal; others get the codes
+ * listed at FX_ERR_DFA_STATE_CAP and FX_ERR_PREFILTER_UNSUPPORTED.
+ * fx_statemap_window_dev: the slab map of window bytes [slab_lo, slab_hi) (window byte 0 is text position `origin`).
+ *   The window must hold min(64, origin + slab_lo) bytes in front of slab_lo (else FX_ERR_BAD_ARGUMENT); it needs no
+ *   look-ahead.  d_map: FX_STATEMAP_MAP_WORDS int64 words = status (0 ok, 1 declined: more than 32 states can arrive at
+ *   the slab, 2 empty slab = the identity), key count, 32 keys (states at the slab's start), 32 end states, 32 last
+ *   accepts (text positions; -1 none, FX_STATEMAP_UNKNOWN: this key's walk could not be decided in the slab).
+ *   d_work: fx_regex_buffer_work_bytes(slab_hi - slab_lo) bytes.
+ * fx_statemap_combine (host-only): chains `nmaps` slab maps in text order from the start state, skipping empty slabs
+ *   and stopping when the state dies, then takes the end-of-text step.  out[0] = end of the match (1-based `to`;
+ *   text_len + 1 when the trailing NUL was consumed; <= 0 none), out[1] = 1 when the scan declined (a slab declined,
+ *   or the true state met an unknown key): answer with the window scan instead.
+ * fx_statemap_back_dev: advances the backward walk held in d_walk (FX_STATEMAP_WALK_WORDS int64 words = position,
+ *   best start so far, reverse state, end of the match).  The caller starts it as {0, 0, FX_STATEMAP_WALK_NEW, out[0]}
+ *   on the GPU that holds text byte end - 1 (the last GPU when end == text_len + 1).  The walk goes as far as the
+ *   window allows; while d_walk[2] != FX_STATEMAP_WALK_DONE it continues on the GPU that holds byte d_walk[0] - 1
+ *   (at most one hand-over per slab the match crosses).  When done, d_walk[0..1] = (from, to): exactly what
+ *   fx_regex_buffer returns for the whole text. */
+#define FX_STATEMAP_MAP_WORDS 98
+#define FX_STATEMAP_UNKNOWN (-2)
+#define FX_STATEMAP_WALK_WORDS 4
+#define FX_STATEMAP_WALK_NEW (-1)
+#define FX_STATEMAP_WALK_DONE (-2)
+int fx_statemap_window_dev(fx_pattern* p, const uint8_t* d_window, int64_t window_len, int64_t slab_lo, int64_t slab_hi,
+                           int64_t origin, int64_t* d_map, void* d_work, void* stream);
+int fx_statemap_combine(const fx_pattern* p, const int64_t* maps, int64_t nmaps, int64_t text_len, int64_t out[2]);
+int fx_statemap_back_dev(fx_pattern* p, const uint8_t* d_window, int64_t window_len, int64_t origin, int64_t text_len,
+                         int64_t* d_walk, void* stream);
 
 /* ---- host-pointer entry points (copy in, run, copy out, synchronous) ------------------- */
 int fx_match_fixed(fx_pattern* p, const uint8_t* buf, int64_t n, int64_t stride, uint8_t* out);
