@@ -1090,6 +1090,9 @@ int launch_finish(fx_pattern* p, const uint8_t* buf, const ScanWindow& W, const 
 //   [6] state-map scan: end of the match, [7] its status (1 = declined)
 //   [8] 1 = the state-map scan has written the answer        [9] 1 = it declined: K4 runs again, without a budget
 //   [12..14] key / undecided / occurrences of that second run
+//   [16..17] presence flags of the prefix / suffix literal (sequential candidate list)
+//   [24..28] fx_regex_buffer_all_dev: the loop's state (rest, count, done, far step wanted, work budget spent)
+//   [30..31] fx_regex_buffer_all_dev: from_to of a far step
 //   from byte 4096: the region maps of the state-map scan (rc, re: 32 x u16 per region; rl: 32 x i64 per region)
 constexpr size_t WORK_HEAD = 4096;
 constexpr int64_t SM_SEG = 32 * (int64_t)SM_SUB;                // one segment: 32 lanes x SM_SUB bytes
@@ -1776,11 +1779,13 @@ int fx_regex_buffer_all_dev(fx_pattern* p, const uint8_t* d_buf, int64_t len, in
     if (len < 0 || capacity < 0 || !count || !d_work || (capacity > 0 && (!d_from || !d_to))) return FX_ERR_BAD_ARGUMENT;
     cudaStream_t s = (cudaStream_t)stream;
     unsigned long long* work = static_cast<unsigned long long*>(d_work);
-    // the loop's own state sits behind the scans' flags in the work area: words [24..27] state, [28..29] from_to of a far step
+    // the loop's own state sits behind the scans' flags in the work area (see WORK_HEAD): words [24..28] state, of which
+    // [28] is the work-budget flag, and [30..31] from_to of a far step.  The two must not overlap: a far match's `from`
+    // in the budget word would turn a loop that then ends in the local step into FX_ERR_WORK_BUDGET.
     int64_t* state = reinterpret_cast<int64_t*>(work + 24);
-    int64_t* ft = reinterpret_cast<int64_t*>(work + 28);
+    int64_t* ft = reinterpret_cast<int64_t*>(work + 30);
     if (p->prog.nfa_engine) return FX_ERR_DFA_STATE_CAP;
-    CUDA_TRY(cudaMemsetAsync(state, 0, 6 * 8, s));
+    CUDA_TRY(cudaMemsetAsync(state, 0, 8 * 8, s));
     Plan pl;
     if ((rc = make_plan(p, pl))) return rc;
     SpanParams sp;

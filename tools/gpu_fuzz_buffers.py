@@ -61,7 +61,8 @@ def main():
             try:
                 f, t, cnt = p.regex_buffer_all(arr, capacity=300)
             except fx.ForgexError as e:
-                assert e.status == 106, (pat, e.status)
+                assert e.status == 106, (pat, e.status)                 # work budget: only where no stand-in exists
+                assert not p.info()["statemap"] or p.info()["literal_prefix_len"] > 0, (seed, pat, "all matches")
                 continue
             got = list(zip(f.tolist(), t.tolist()))
             assert got[:len(want)] == want[:len(got)] and len(got) >= min(len(want), 300), (seed, pat, got[:3], want[:3], cnt, len(want))
