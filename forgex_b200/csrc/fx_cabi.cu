@@ -69,10 +69,6 @@ struct FirstSet {
     bool two = false;            // one first byte, and after it one ASCII byte (plus, maybe, lead bytes) keeps the automaton alive
     uint8_t second = 0;
     bool second_high = false;
-    // any first byte of F, and after it at most two ASCII byte values (plus, maybe, lead bytes) keep the automaton alive
-    bool set2 = false;
-    uint8_t set2_a = 0, set2_b = 0;
-    bool set2_high = false;
 };
 
 }  // namespace
@@ -149,7 +145,8 @@ bool prefilter_is_neutral(const fx::Program& anchored) {
     return true;
 }
 
-// tuning knobs for experiments (environment, read per launch)
+// route overrides (environment, read per call): tests and tools force a kernel or a path that the default choice
+// would not take for their input, to check it against the oracle.  DESIGN.md lists them.
 int env_int(const char* name, int dflt) {
     const char* v = getenv(name);
     return v && *v ? atoi(v) : dflt;
@@ -206,32 +203,6 @@ bool sparse_first_set(const fx::ByteTable& at, FirstSet& fs, bool for_in) {
                 else hi2 = true;
             }
             if (nascii == 1 && v2 != 0 && !cont) { fs.two = true; fs.second = (uint8_t)v2; fs.second_high = hi2; }
-        }
-    }
-    // the same for byte SETS (the long-buffer sweep): every first byte steps into a plain state (no accept, no
-    // sequence), and the union of what may follow is at most two ASCII values != NUL, no continuation byte
-    {
-        bool ok = true, follow[256];
-        for (int c = 0; c < 256; c++) follow[c] = false;
-        for (int b1 = 0; b1 < 128 && ok; b1++) {           // (lead bytes as first bytes enter a sequence: the filter lets them pass)
-            if (!in_f[b1]) continue;
-            const uint16_t w1 = at.table[((size_t)at.q0 << at.row_shift) + at.classmap[b1]];
-            if ((w1 & (fxk::W_ACC | fxk::W_INTER)) != 0 || (w1 & fxk::W_STATE) == 0) { ok = false; break; }
-            for (int c = 0; c < 256; c++) {
-                const uint16_t w2 = at.table[((size_t)(w1 & fxk::W_STATE) << at.row_shift) + at.classmap[c]];
-                if ((w2 & (fxk::W_STATE | fxk::W_ACC)) != 0) follow[c] = true;
-            }
-        }
-        int nascii = 0, v[2] = {0, 0};
-        bool cont = false, hi2 = false;
-        for (int c = 0; c < 256 && ok; c++) {
-            if (!follow[c]) continue;
-            if (c < 0x80) { if (nascii < 2) v[nascii] = c; nascii++; }
-            else if (c < 0xC0) cont = true;
-            else hi2 = true;
-        }
-        if (ok && nascii >= 1 && nascii <= 2 && !cont && v[0] != 0 && (nascii == 1 || v[1] != 0)) {
-            fs.set2 = true; fs.set2_a = (uint8_t)v[0]; fs.set2_b = (uint8_t)(nascii == 2 ? v[1] : v[0]); fs.set2_high = hi2;
         }
     }
     return true;
@@ -350,8 +321,8 @@ int make_plan(fx_pattern* p, Plan& pl) {
     const DeviceTables& d = p->dev;
     const bool span = bt.flag_bits;
     int classed_bytes = (int)bt.table.size() * 2, direct_bytes = (int)bt.direct.size() * 2;
-    bool direct16_ok = span && d.direct != nullptr && direct_bytes <= env_int("FX_DIRECT_LIMIT_BYTES", DIRECT_LIMIT_BYTES);
-    bool direct8_ok = !span && d.table8 != nullptr && env_int("FX_USE_TABLE8", 1);
+    bool direct16_ok = span && d.direct != nullptr && direct_bytes <= DIRECT_LIMIT_BYTES;
+    bool direct8_ok = !span && d.table8 != nullptr;
     bool classed_smem_ok = classed_bytes <= SMEM_TABLE_LIMIT_BYTES;
     int res = p->residency;
     if (res == FX_TABLE_SMEM && !direct16_ok && !direct8_ok && !classed_smem_ok) return FX_ERR_BAD_ARGUMENT;
@@ -454,35 +425,6 @@ int launch_nfa_regex(fx_pattern* p, const uint8_t* buf, const int64_t* off, int6
     return cuda_status(cudaGetLastError());
 }
 
-// A table that is read from global memory (FX_TABLE_GLOBAL, or too big for shared memory) is marked PERSISTING in L2
-// for the launches that walk it: the text streams through L2 at terabytes per second and would otherwise keep evicting
-// table lines.  Best effort (errors are ignored: the window is a hint); cleared again behind the launch.
-struct L2Window {
-    cudaStream_t s;
-    bool set = false;
-    L2Window(cudaStream_t stream, const void* base, size_t bytes) : s(stream) {
-        if (!base || bytes == 0 || !env_int("FX_L2_PERSIST", 1)) return;
-        static std::once_flag once;
-        std::call_once(once, [] { cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 4 << 20); cudaGetLastError(); });
-        cudaStreamAttrValue v;
-        memset(&v, 0, sizeof(v));
-        v.accessPolicyWindow.base_ptr = const_cast<void*>(base);
-        v.accessPolicyWindow.num_bytes = bytes;
-        v.accessPolicyWindow.hitRatio = 1.0f;
-        v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        v.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        set = cudaStreamSetAttribute(s, cudaStreamAttributeAccessPolicyWindow, &v) == cudaSuccess;
-        cudaGetLastError();
-    }
-    ~L2Window() {
-        if (!set) return;
-        cudaStreamAttrValue v;
-        memset(&v, 0, sizeof(v));
-        cudaStreamSetAttribute(s, cudaStreamAttributeAccessPolicyWindow, &v);
-        cudaGetLastError();
-    }
-};
-
 // ---- launchers -----------------------------------------------------------------------------
 inline size_t staged_bytes(const Plan& pl) { return (size_t)((pl.table_bytes + 15) & ~15); }
 
@@ -551,7 +493,6 @@ int launch_fixed(fx_pattern* p, const uint8_t* buf, int64_t n, int64_t stride, u
         if (rc2) return rc2;
         long long want = (n + 1023) / 1024, cap = (long long)p->dev.sm_count * bps * 2;
         const int grid = (int)(want < cap ? want : cap);
-        L2Window keep(s, in_smem ? nullptr : p->dev.ctab4, (size_t)p->prog.bt.nstates * 8);
         if (in_smem) kern_s<<<grid, 1024, smem, s>>>(pl.kp, p->dev.ctab4, p->dev.cmap4, buf, n, stride, out);
         else kern_g<<<grid, 1024, smem, s>>>(pl.kp, p->dev.ctab4, p->dev.cmap4, buf, n, stride, out);
         g_launches++;
@@ -561,12 +502,11 @@ int launch_fixed(fx_pattern* p, const uint8_t* buf, int64_t n, int64_t stride, u
     }
     if (pl.kind == 0) return launch_fixed_v<OP, 0>(p, pl, buf, n, stride, out, s, generic);
     if (pl.kind == 2) return launch_fixed_v<OP, 2>(p, pl, buf, n, stride, out, s, generic);
-    L2Window keep(s, p->dev.table, p->prog.bt.table.size() * 2);
     return launch_fixed_v<OP, 3>(p, pl, buf, n, stride, out, s, generic);
 }
 
 // tiles of `spt` consecutive strings; up to `cap` bytes of a tile's text are staged in shared memory.  The tile is
-// sized so that `ctas_per_sm` CTAs fit one SM's shared memory (227 KB usable, 1 KB reserved per CTA).
+// sized so that 4 CTAs fit one SM's shared memory (227 KB usable, 1 KB reserved per CTA).
 struct Tiling {
     int spt, cap;
     int64_t ntiles;
@@ -579,8 +519,7 @@ Tiling make_tiling(const Plan& pl, int64_t n, int64_t total, int extra = 0, int6
     int64_t avg = n > 0 ? (total + n - 1) / n : 1;
     if (avg < 1) avg = 1;
     t.table_smem = (int)staged_bytes(pl);
-    int ctas = env_int("FX_CTAS_PER_SM", 4);
-    int64_t per_cta = (227 * 1024) / ctas - 1024;
+    const int64_t per_cta = (227 * 1024) / 4 - 1024;
     // strings per tile: about one per thread, fewer when strings are long, more when they are short
     int64_t spt = 0, cap = 0;
     for (int iter = 0; iter < 2; iter++) {
@@ -594,7 +533,6 @@ Tiling make_tiling(const Plan& pl, int64_t n, int64_t total, int extra = 0, int6
         if (spt < 32) spt = 32;
         if (spt > 2048) spt = 2048;
     }
-    spt = env_int("FX_TILE_STRINGS", (int)spt);
     t.spt = (int)spt;
     t.cap = (int)cap;
     t.ntiles = (n + spt - 1) / spt;
@@ -618,67 +556,15 @@ int launch_ragged_t(fx_pattern* p, const Plan& pl, const uint8_t* buf, const int
     return cuda_status(cudaGetLastError());
 }
 
-template <int OP, int KIND>
-int launch_pairs_t(fx_pattern* p, const Plan& pl, const uint8_t* buf, const int64_t* off, int64_t n, int64_t total,
-                   uint8_t* out, cudaStream_t s) {
-    auto kern = k_bool_ragged_pairs<OP, KIND>;
-    int table_smem = (int)staged_bytes(pl);
-    int64_t avg = n > 0 ? (total + n - 1) / n : 1;
-    if (avg < 1) avg = 1;
-    int ctas = env_int("FX_CTAS_PER_SM", 4);
-    int64_t per_cta = (227 * 1024) / ctas - 1024;
-    int64_t cap = per_cta - (tile_offset_pairs(table_smem, 256) + 64 + 128);
-    if (cap < 8192) cap = 8192;
-    cap &= ~(int64_t)127;
-    int64_t spt = (cap * 4 / 5) / avg;
-    spt = (spt / 32) * 32;
-    if (spt < 32) spt = 32;
-    if (spt > 256) spt = 256;
-    spt = env_int("FX_TILE_STRINGS", (int)spt);
-    if (spt > 256) spt = 256;
-    size_t smem = (size_t)tile_offset_pairs(table_smem, (int)spt) + (size_t)cap + 64;
-    int64_t ntiles = (n + spt - 1) / spt;
-    int bps = 0;
-    int rc = occupancy_grid(kern, 128, smem, p->dev.sm_count, bps);
-    if (rc) return rc;
-    long long capg = (long long)p->dev.sm_count * bps;
-    int grid = (int)(ntiles < capg ? ntiles : capg);
-    if (grid < 1) grid = 1;
-    kern<<<grid, 128, smem, s>>>(pl.kp, buf, off, n, total, out, (int)spt, (int)cap, ntiles, table_smem);
-    g_launches++;
-    return cuda_status(cudaGetLastError());
-}
-
-template <int OP, int KIND>
-int launch_stream_t(fx_pattern* p, const Plan& pl, const uint8_t* buf, const int64_t* off, int64_t n, int64_t total,
-                    uint8_t* out, cudaStream_t s) {
-    auto kern = k_bool_stream<OP, KIND>;
-    size_t smem = 256 + staged_bytes(pl);
-    int bps = 0;
-    int rc = occupancy_grid(kern, 256, smem, p->dev.sm_count, bps);
-    if (rc) return rc;
-    int window = env_int("FX_WINDOW", 1024);
-    if (window < 64) window = 64;
-    int64_t nwindows = total / window + 1;
-    long long want = (nwindows + 255) / 256;
-    long long cap = (long long)p->dev.sm_count * bps;
-    int grid = (int)(want < cap ? want : cap);
-    if (grid < 1) grid = 1;
-    kern<<<grid, 256, smem, s>>>(pl.kp, buf, off, n, total, out, window, nwindows);
-    g_launches++;
-    return cuda_status(cudaGetLastError());
-}
-
 // K2c: a warp sweeps tiles of `spt` consecutive strings, about 24 KB of text each
-template <int KIND, int NR, bool HIGH, bool TWO, int MINB, int ROWS>
-int launch_sparse_v(fx_pattern* p, const Plan& pl, const SparseParams& sp, int table_bytes, const uint8_t* buf,
+template <int KIND, int NR, bool HIGH, bool TWO>
+int launch_sparse_t(fx_pattern* p, const Plan& pl, const SparseParams& sp, int table_bytes, const uint8_t* buf,
                     const int64_t* off, int64_t n, int64_t total, uint8_t* out, cudaStream_t s, int64_t stride) {
-    auto kern = k_in_sparse<KIND, NR, HIGH, TWO, MINB, ROWS>;
+    auto kern = k_in_sparse<KIND, NR, HIGH, TWO>;
     int64_t avg = n > 0 ? (total + n - 1) / n : 1;
     if (avg < 1) avg = 1;
-    int64_t want = env_int("FX_SPARSE_TILE_BYTES", 24 * 1024) / avg;    // (one sweep segment holds 32 KB)
-    int spt = (int)(want < 32 ? 32 : want > 4096 ? 4096 : want);
-    spt = env_int("FX_TILE_STRINGS", spt);
+    int64_t want = (24 * 1024) / avg;       // (one sweep segment holds 32 KB)
+    const int spt = (int)(want < 32 ? 32 : want > 4096 ? 4096 : want);
     const int64_t ntiles = (n + spt - 1) / spt;
     const int table_smem = KIND == 3 ? 0 : (table_bytes + 15) & ~15;
     const size_t smem = (size_t)sparse_shared_head(table_smem) + 8 * (size_t)SPARSE_WARP_BYTES;
@@ -693,17 +579,9 @@ int launch_sparse_v(fx_pattern* p, const Plan& pl, const SparseParams& sp, int t
     // phase: every result is "false unless a start wins", so the results are cleared here, at copy speed
     const int prezeroed = sp.start_nul == 0 && pl.kp.q0_accepting == 0;
     if (prezeroed) CUDA_TRY(cudaMemsetAsync(out, 0, (size_t)n, s));
-    kern<<<grid, 256, smem, s>>>(pl.kp, sp, buf, off, n, total, out, spt, ntiles, table_smem, prezeroed, env_int("FX_SPARSE_FLUSH", 0),
-                                   env_int("FX_SPARSE_STREAM_HINT", 1), stride);
+    kern<<<grid, 256, smem, s>>>(pl.kp, sp, buf, off, n, total, out, spt, ntiles, table_smem, prezeroed, stride);
     g_launches++;
     return cuda_status(cudaGetLastError());
-}
-
-template <int KIND, int NR, bool HIGH, bool TWO>
-int launch_sparse_t(fx_pattern* p, const Plan& pl, const SparseParams& sp, int table_bytes, const uint8_t* buf,
-                    const int64_t* off, int64_t n, int64_t total, uint8_t* out, cudaStream_t s, int64_t stride) {
-    // 4 CTAs per SM, 4 rows (4 KB per warp) in flight: the best of the measured combinations (DESIGN.md section 5)
-    return launch_sparse_v<KIND, NR, HIGH, TWO, 4, 4>(p, pl, sp, table_bytes, buf, off, n, total, out, s, stride);
 }
 
 template <int KIND, bool HIGH>
@@ -711,7 +589,7 @@ int launch_sparse_k(fx_pattern* p, const Plan& pl, const SparseParams& sp, int t
                     int64_t n, int64_t total, uint8_t* out, cudaStream_t s, int64_t stride) {
     if (p->first.sweep_nr == 1 && p->first.sweep_lo[0] == p->first.sweep_hi[0]) {      // one byte value: the cheaper zero-byte test
         const SparseParams& one = sp;      // (fill_sweep has put the byte value into add_lo[0])
-        if (p->first.two && env_int("FX_SPARSE_TWO", 1)) return launch_sparse_t<KIND, -1, HIGH, true>(p, pl, one, tb, buf, off, n, total, out, s, stride);
+        if (p->first.two) return launch_sparse_t<KIND, -1, HIGH, true>(p, pl, one, tb, buf, off, n, total, out, s, stride);
         return launch_sparse_t<KIND, -1, HIGH, false>(p, pl, one, tb, buf, off, n, total, out, s, stride);
     }
     switch (p->first.sweep_nr) {
@@ -732,13 +610,6 @@ void fill_sweep(const FirstSet& f, SparseParams& sp) {
     if (f.sweep_nr == 1 && f.sweep_lo[0] == f.sweep_hi[0]) sp.add_lo[0] = f.sweep_lo[0] * 0x01010101u;   // NR = -1 form
     sp.second = f.second * 0x01010101u;
     sp.second_high = f.second_high ? 0xFFFFFFFFu : 0u;
-    sp.second_b = sp.second;
-}
-// the SET2 form of the long-buffer sweep
-void fill_sweep_set2(const FirstSet& f, SparseParams& sp) {
-    sp.second = f.set2_a * 0x01010101u;
-    sp.second_b = f.set2_b * 0x01010101u;
-    sp.second_high = f.set2_high ? 0x80808080u : 0u;
 }
 
 int launch_sparse(fx_pattern* p, const Plan& pl, const uint8_t* buf, const int64_t* off, int64_t n, int64_t total,
@@ -752,7 +623,7 @@ int launch_sparse(fx_pattern* p, const Plan& pl, const uint8_t* buf, const int64
     sp.q0 = at.q0; sp.start_nul = at.start_nul;
     fill_sweep(p->first, sp);
     const int tb = (int)at.table.size() * 2;
-    const bool smem_table = p->residency != FX_TABLE_GLOBAL && tb <= env_int("FX_SPARSE_SMEM_TABLE_BYTES", 24 * 1024);
+    const bool smem_table = p->residency != FX_TABLE_GLOBAL && tb <= 24 * 1024;
     if (smem_table)
         return p->first.high ? launch_sparse_k<2, true>(p, pl, sp, tb, buf, off, n, total, out, s, stride)
                              : launch_sparse_k<2, false>(p, pl, sp, tb, buf, off, n, total, out, s, stride);
@@ -774,16 +645,6 @@ int launch_ragged(fx_pattern* p, const uint8_t* buf, const int64_t* off, int64_t
     if (OP == 1 && !generic && p->sparse && n < (1ll << 31) && env_int("FX_SPARSE", 1)) {      // sparse starts (K2c)
         p->last_sparse = 1;
         return launch_sparse(p, pl, buf, off, n, total, out, s, 0);
-    }
-    if (!generic && env_int("FX_RAGGED_FORM", 0) == 2) {      // length-balanced pairs (K2p)
-        if (pl.kind == 0) return launch_pairs_t<OP, 0>(p, pl, buf, off, n, total, out, s);
-        if (pl.kind == 2) return launch_pairs_t<OP, 2>(p, pl, buf, off, n, total, out, s);
-        return launch_pairs_t<OP, 3>(p, pl, buf, off, n, total, out, s);
-    }
-    if (!generic && env_int("FX_RAGGED_FORM", 0) == 1) {      // streaming form (K2s)
-        if (pl.kind == 0) return launch_stream_t<OP, 0>(p, pl, buf, off, n, total, out, s);
-        if (pl.kind == 2) return launch_stream_t<OP, 2>(p, pl, buf, off, n, total, out, s);
-        return launch_stream_t<OP, 3>(p, pl, buf, off, n, total, out, s);
     }
     if (pl.kind == 0) return launch_ragged_t<OP, 0>(p, pl, buf, off, n, total, out, s, generic);
     if (pl.kind == 2) return launch_ragged_t<OP, 2>(p, pl, buf, off, n, total, out, s, generic);
@@ -821,16 +682,16 @@ void fill_span_params(fx_pattern* p, SpanParams& sp) {
     sp.nmixed = (int)(rv.mixed.size() / 64);
 }
 
-template <int FK, bool RS, int WARPS>
-int launch_span_w(fx_pattern* p, const Plan& pl, const SpanParams& sp, int fwd_bytes, const uint8_t* buf,
+template <int FK, bool RS>
+int launch_span_t(fx_pattern* p, const Plan& pl, const SpanParams& sp, int fwd_bytes, const uint8_t* buf,
                   const int64_t* off, int64_t n, int64_t total, int64_t* from, int64_t* to, cudaStream_t s) {
-    auto kern = k_span_ragged<FK, RS, WARPS>;
-    // one CTA of WARPS warps per SM; every warp stages its own tiles: the tables take their share of the SM's
+    auto kern = k_span_ragged<FK, RS>;
+    // one CTA of SPAN_WARPS warps per SM; every warp stages its own tiles: the tables take their share of the SM's
     // shared memory once, the rest is divided among the warps
     int64_t avg = n > 0 ? (total + n - 1) / n : 1;
     if (avg < 1) avg = 1;
     const SpanHead H = span_head(fwd_bytes, sp.rstates * sp.rclasses * 2, sp.nmixed, RS);
-    int per_warp = ((227 * 1024 - 1024 - H.bytes) / WARPS) & ~127;
+    int per_warp = ((227 * 1024 - 1024 - H.bytes) / SPAN_WARPS) & ~127;
     if (per_warp < 1024) return FX_ERR_BAD_ARGUMENT;
     int cap = per_warp, spt = 1;
     for (;;) {
@@ -839,72 +700,19 @@ int launch_span_w(fx_pattern* p, const Plan& pl, const SpanParams& sp, int fwd_b
         if (cap <= 512 || span_layout(spt, cap).warp_bytes <= per_warp) break;
         cap -= 128;
     }
-    spt = env_int("FX_TILE_STRINGS", spt);
-    if (spt > 512) spt = 512;
     while (spt > 1 && span_layout(spt, cap).warp_bytes > per_warp) spt--;
     const int64_t ntiles = (n + spt - 1) / spt;
-    const size_t smem = (size_t)H.bytes + (size_t)WARPS * (size_t)span_layout(spt, cap).warp_bytes;
+    const size_t smem = (size_t)H.bytes + (size_t)SPAN_WARPS * (size_t)span_layout(spt, cap).warp_bytes;
     int bps = 0;
-    int rc = occupancy_grid(kern, WARPS * 32, smem, p->dev.sm_count, bps);
+    int rc = occupancy_grid(kern, SPAN_WARPS * 32, smem, p->dev.sm_count, bps);
     if (rc) return rc;
     long long capg = (long long)p->dev.sm_count * bps;
-    long long want = (ntiles + WARPS - 1) / WARPS;
+    long long want = (ntiles + SPAN_WARPS - 1) / SPAN_WARPS;
     int grid = (int)(want < capg ? want : capg);
     if (grid < 1) grid = 1;
-    int round_bytes = env_int("FX_SPAN_ROUND", SPAN_ROUND) & ~3;
-    if (round_bytes < 4) round_bytes = 4;
-    kern<<<grid, WARPS * 32, smem, s>>>(pl.kp, sp, buf, off, n, total, from, to, spt, cap, ntiles, fwd_bytes, round_bytes);
+    kern<<<grid, SPAN_WARPS * 32, smem, s>>>(pl.kp, sp, buf, off, n, total, from, to, spt, cap, ntiles, fwd_bytes);
     g_launches++;
     return cuda_status(cudaGetLastError());
-}
-
-template <int FK, bool RS>
-int launch_span_t(fx_pattern* p, const Plan& pl, const SpanParams& sp, int fwd_bytes, const uint8_t* buf,
-                  const int64_t* off, int64_t n, int64_t total, int64_t* from, int64_t* to, cudaStream_t s) {
-    // (experiment, FX_SPAN_WARPS=24: fewer warps, larger tiles per warp)
-    if (env_int("FX_SPAN_WARPS", SPAN_WARPS) == 24) return launch_span_w<FK, RS, 24>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s);
-    return launch_span_w<FK, RS, SPAN_WARPS>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s);
-}
-
-// K3f, streaming form: every warp owns a ring of RING_NB small buffers and never waits for a tile to finish
-template <int FK, bool RS, int WARPS>
-int launch_span_stream_t(fx_pattern* p, const Plan& pl, const SpanParams& sp, int fwd_bytes, const uint8_t* buf,
-                         const int64_t* off, int64_t n, int64_t total, int64_t* from, int64_t* to, cudaStream_t s) {
-    auto kern = k_span_stream<FK, RS, WARPS>;
-    int64_t avg = n > 0 ? (total + n - 1) / n : 1;
-    if (avg < 1) avg = 1;
-    const SpanHead H = span_head(fwd_bytes, sp.rstates * sp.rclasses * 2, sp.nmixed, RS);
-    const int per_buf = (((227 * 1024 - 1024 - H.bytes) / WARPS) / RING_NB) & ~127;
-    if (per_buf < 512) return FX_ERR_BAD_ARGUMENT;
-    int cap = per_buf, spt = 1;
-    for (;;) {
-        int64_t want = ((int64_t)cap * 7 / 8) / avg;       // expect the tile to fill most of the staged capacity
-        spt = (int)(want < 1 ? 1 : want > 512 ? 512 : want);
-        if (cap <= 256 || ring_layout(spt, cap).buf_bytes <= per_buf) break;
-        cap -= 128;
-    }
-    spt = env_int("FX_TILE_STRINGS", spt);
-    if (spt > 512) spt = 512;
-    while (spt > 1 && ring_layout(spt, cap).buf_bytes > per_buf) spt--;
-    const int64_t ntiles = (n + spt - 1) / spt;
-    const size_t smem = (size_t)H.bytes + (size_t)WARPS * RING_NB * (size_t)ring_layout(spt, cap).buf_bytes;
-    int bps = 0;
-    int rc = occupancy_grid(kern, WARPS * 32, smem, p->dev.sm_count, bps);
-    if (rc) return rc;
-    long long capg = (long long)p->dev.sm_count * bps;
-    long long want = (ntiles + WARPS - 1) / WARPS;
-    int grid = (int)(want < capg ? want : capg);
-    if (grid < 1) grid = 1;
-    kern<<<grid, WARPS * 32, smem, s>>>(pl.kp, sp, buf, off, n, total, from, to, spt, cap, ntiles, fwd_bytes);
-    g_launches++;
-    return cuda_status(cudaGetLastError());
-}
-template <int FK, bool RS>
-int launch_span_stream(fx_pattern* p, const Plan& pl, const SpanParams& sp, int fwd_bytes, const uint8_t* buf,
-                       const int64_t* off, int64_t n, int64_t total, int64_t* from, int64_t* to, cudaStream_t s) {
-    // 16 warps per SM: the walker state (ring bookkeeping + a forward walk + a backward job) needs ~110 registers; with
-    // 32 warps (64 registers) ptxas spills 400 bytes per thread
-    return launch_span_stream_t<FK, RS, 16>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s);
 }
 
 int launch_regex_ragged(fx_pattern* p, const uint8_t* buf, const int64_t* off, int64_t n, int64_t total,
@@ -926,14 +734,6 @@ int launch_regex_ragged(fx_pattern* p, const uint8_t* buf, const int64_t* off, i
         if (fk == 0 && !p->dev.sp_direct) fk = 1;
         const int fwd_bytes = fk == 0 ? st.nstates * SPAN_ROW * 2 : fk == 1 ? classed_bytes : 0;
         const bool rs = !rv.page.empty() && (int)(rv.delta16.size() * 2 + 1024 + rv.mixed.size()) <= SPAN_REV_SMEM_BYTES;
-        if (env_int("FX_SPAN_STREAM", 0)) {        // experiment: ring of buffers per warp, continuous claiming (lost, see DESIGN.md)
-            if (fk == 0) return rs ? launch_span_stream<0, true>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s)
-                                   : launch_span_stream<0, false>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s);
-            if (fk == 1) return rs ? launch_span_stream<1, true>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s)
-                                   : launch_span_stream<1, false>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s);
-            return rs ? launch_span_stream<2, true>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s)
-                      : launch_span_stream<2, false>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s);
-        }
         if (fk == 0) return rs ? launch_span_t<0, true>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s)
                                : launch_span_t<0, false>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s);
         if (fk == 1) return rs ? launch_span_t<1, true>(p, pl, sp, fwd_bytes, buf, off, n, total, from, to, s)
@@ -965,11 +765,11 @@ int launch_scan_t(fx_pattern* p, const Plan& pl, const uint8_t* buf, const ScanW
     return cuda_status(cudaGetLastError());
 }
 
-template <int KIND, int NR, bool HIGH, bool PREFIX, bool SET2 = false>
+template <int KIND, int NR, bool HIGH, bool PREFIX>
 int launch_scan_sparse_t(fx_pattern* p, const Plan& pl, const SparseParams& sp, const uint8_t* buf, const ScanWindow& W,
                          unsigned long long* best, cudaStream_t s, const unsigned long long* gate,
-                         const unsigned long long* run_if = nullptr, ScanBudget budget = ScanBudget{nullptr, nullptr, 0ull, 0}) {
-    auto kern = k_buffer_scan_sparse<KIND, NR, HIGH, PREFIX, SET2>;
+                         const unsigned long long* run_if, ScanBudget budget) {
+    auto kern = k_buffer_scan_sparse<KIND, NR, HIGH, PREFIX>;
     int table_smem = (int)staged_bytes(pl);
     size_t smem = (size_t)scan_sparse_smem_bytes(table_smem);
     int bps = 0;
@@ -980,8 +780,7 @@ int launch_scan_sparse_t(fx_pattern* p, const Plan& pl, const SparseParams& sp, 
     long long cap = (long long)p->dev.sm_count * bps;
     int grid = (int)(want < cap ? want : cap);
     if (grid < 1) grid = 1;
-    budget.flags = env_int("FX_K4_FLAGS", 0);
-    kern<<<grid, 256, smem, s>>>(pl.kp, sp, buf, W, best, table_smem, gate, env_int("FX_K4_PHASES", 3) | (env_int("FX_K4_LOAD", 1) << 4), run_if, budget);
+    kern<<<grid, 256, smem, s>>>(pl.kp, sp, buf, W, best, table_smem, gate, run_if, budget);
     g_launches++;
     return cuda_status(cudaGetLastError());
 }
@@ -994,17 +793,6 @@ int launch_scan_sparse(fx_pattern* p, const Plan& pl, const uint8_t* buf, const 
     fill_sweep(p->first, sp);
     const FirstSet& f = p->first;
     const bool one = f.sweep_nr == 1 && f.sweep_lo[0] == f.sweep_hi[0];
-    // the two-byte test of the unit phase (the follower of a unit's last byte is never assumed)
-    // (measured on C4: 15.2 vs 13.1 ms for 32 GiB -- the test costs ~80 instructions per queued unit and saves fewer: off)
-    if (f.set2 && f.sweep_nr >= 1 && f.sweep_nr <= 2 && env_int("FX_SWEEP_SET2", 0)) {
-        fill_sweep_set2(f, sp);
-        if (one) return f.high ? launch_scan_sparse_t<KIND, -1, true, false, true>(p, pl, sp, buf, W, best, s, gate, run_if, bg)
-                               : launch_scan_sparse_t<KIND, -1, false, false, true>(p, pl, sp, buf, W, best, s, gate, run_if, bg);
-        if (f.sweep_nr == 1) return f.high ? launch_scan_sparse_t<KIND, 1, true, false, true>(p, pl, sp, buf, W, best, s, gate, run_if, bg)
-                                           : launch_scan_sparse_t<KIND, 1, false, false, true>(p, pl, sp, buf, W, best, s, gate, run_if, bg);
-        return f.high ? launch_scan_sparse_t<KIND, 2, true, false, true>(p, pl, sp, buf, W, best, s, gate, run_if, bg)
-                      : launch_scan_sparse_t<KIND, 2, false, false, true>(p, pl, sp, buf, W, best, s, gate, run_if, bg);
-    }
     if (f.sweep_nr == 0) return launch_scan_sparse_t<KIND, 0, true, false>(p, pl, sp, buf, W, best, s, gate, run_if, bg);
     if (one) return f.high ? launch_scan_sparse_t<KIND, -1, true, false>(p, pl, sp, buf, W, best, s, gate, run_if, bg)
                            : launch_scan_sparse_t<KIND, -1, false, false>(p, pl, sp, buf, W, best, s, gate, run_if, bg);
@@ -1033,7 +821,7 @@ int launch_scan_prefix(fx_pattern* p, const Plan& pl, const uint8_t* buf, const 
 enum { SCAN_AUTO = 0, SCAN_ALL = 1 };
 int launch_scan(fx_pattern* p, const uint8_t* buf, const ScanWindow& W, unsigned long long* best, cudaStream_t s,
                 int mode = SCAN_AUTO, const unsigned long long* gate = nullptr, const unsigned long long* run_if = nullptr,
-                ScanBudget bg = ScanBudget{nullptr, nullptr, 0ull, 0}) {
+                ScanBudget bg = ScanBudget{nullptr, nullptr, 0ull}) {
     if (W.len < 0 || W.start_lo < 0 || W.start_hi > W.len || W.start_lo > W.start_hi) return FX_ERR_BAD_ARGUMENT;
     if (p->prog.nfa_engine) return FX_ERR_DFA_STATE_CAP;        // the window forms need the table engine
     const bool prefixed = p->prog.prefix_active && !p->prog.literal_only;
@@ -1222,7 +1010,7 @@ int launch_buffer(fx_pattern* p, const uint8_t* buf, int64_t len, int64_t* from_
         // winner begins with the literal's own bytes (the prefilter is provably neutral for this pattern: every match
         // begins with the literal's code points; only an overlong encoding of them could differ).  If the winner does
         // not, or the scan declines, the candidate scan runs again without a budget.
-        ScanBudget bg{work + 5, work + 4, (unsigned long long)len * 16ull + (4ull << 20), 0};
+        ScanBudget bg{work + 5, work + 4, (unsigned long long)len * 16ull + (4ull << 20)};
         int rc = sm_mode == 2 ? FX_OK : launch_scan(p, buf, W, best, s, SCAN_AUTO, nullptr, nullptr, bg);
         if (rc) return rc;
         if (sm_mode == 2) CUDA_TRY(cudaMemsetAsync(work + 4, 0x01, 1, s));
@@ -1237,7 +1025,7 @@ int launch_buffer(fx_pattern* p, const uint8_t* buf, int64_t len, int64_t* from_
         const bool k4_first = p->sparse && p->first.sweep_nr <= 2 && env_int("FX_SPARSE", 1) && sm_mode != 2;
         int rc;
         if (k4_first) {
-            ScanBudget bg{work + 5, work + 4, (unsigned long long)len * 16ull + (4ull << 20), 0};
+            ScanBudget bg{work + 5, work + 4, (unsigned long long)len * 16ull + (4ull << 20)};
             rc = launch_scan(p, buf, W, best, s, SCAN_AUTO, nullptr, nullptr, bg);
             if (rc) return rc;
         } else {
@@ -1253,9 +1041,9 @@ int launch_buffer(fx_pattern* p, const uint8_t* buf, int64_t len, int64_t* from_
     // What is left: patterns without the span path (a cap was passed), and prefix literals that are not provably neutral.
     // The candidate scan still runs under the work budget; without a linear-time stand-in a spent budget is reported as
     // (-2, -2) = FX_ERR_WORK_BUDGET instead of occupying the GPU with the reference's quadratic loop.
-    ScanBudget bg{work + 5, work + 4, (unsigned long long)len * 16ull + (4ull << 20), 0};
+    ScanBudget bg{work + 5, work + 4, (unsigned long long)len * 16ull + (4ull << 20)};
     const bool budgeted = env_int("FX_STATEMAP", 1) != 0;
-    if (!budgeted) bg = ScanBudget{nullptr, nullptr, 0ull, 0};
+    if (!budgeted) bg = ScanBudget{nullptr, nullptr, 0ull};
     if (len >= 1) {
         int rc = launch_scan(p, buf, W, best, s, SCAN_AUTO, nullptr, nullptr, bg);
         if (rc) return rc;

@@ -68,19 +68,14 @@ __device__ __forceinline__ uint4 ldg_nc_v4(const void* p) {  // streaming 16-byt
     asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
     return r;
 }
-// The sweep load of K4 under a choice of cache policies (FX_K4_LOAD): 0 = no L1 allocation (the K2c choice), 1 = plain
-// read-only load, allocating in L1 (K4's default), 2 = L1 evict_last, 3 = no L1 allocation + L2 evict_last, 4 = no L1
-// allocation + 256-byte L2 prefetch.  Measured on C4 (profiles/r02_prof_c4_sweep_load_policy.txt): under policy 0 the
-// unit phase's re-read of a candidate unit, microseconds after the sweep read it, MISSES L2 and goes to DRAM at 64-byte
-// granularity -- 3.55 GB of DRAM reads for 2.15 GB of text; policies 1-3 bring that to 2.34 GB and the search from
-// 3.43 to 3.27 ms per 8 GiB.
-__device__ __forceinline__ uint4 ldg_v4_policy(const void* p, int lp, unsigned long long pol) {
+// The sweep load of K4: a plain read-only load that allocates in L1.  Measured on C4
+// (profiles/r02_prof_c4_sweep_load_policy.txt): with no L1 allocation (ldg_nc_v4, the K2c choice) the unit phase's
+// re-read of a candidate unit, microseconds after the sweep read it, MISSES L2 and goes to DRAM at 64-byte granularity
+// -- 3.55 GB of DRAM reads for 2.15 GB of text; this load brings that to 2.34 GB and the search from 3.43 to 3.27 ms
+// per 8 GiB.
+__device__ __forceinline__ uint4 ldg_v4(const void* p) {
     uint4 r;
-    if (lp == 1) asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-    else if (lp == 2) asm volatile("ld.global.nc.L1::evict_last.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-    else if (lp == 3) asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p), "l"(pol));
-    else if (lp == 4) asm volatile("ld.global.nc.L1::no_allocate.L2::256B.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-    else asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
+    asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
     return r;
 }
 __device__ __forceinline__ uint2 ldg_nc_v2(const void* p) {
@@ -954,7 +949,6 @@ struct SparseParams {
     uint32_t add_hi[4];         // (0x7F - hi) * 0x01010101: bit 7 of (y + add_hi) <=> y >  hi
     uint32_t second;            // TWO: the one ASCII byte that keeps the automaton alive after the first, in all four bytes
     uint32_t second_high;       // TWO: 0xFFFFFFFF when bytes >= 0xC0 keep it alive as well (lead bytes), else 0
-    uint32_t second_b;          // SET2 (long-buffer sweep): a second possible follower (== second when there is only one)
 };
 
 // shared memory of K2c: classmap 256 | table | pad to 16 | 8 warps x (unit queue 64 x uint4 | start queue 64 x uint4)
@@ -1012,25 +1006,6 @@ __device__ __forceinline__ uint32_t unit_any(const SparseParams& sp, const uint4
         for (int k = 0; k < 8; k++) any |= first_mask<NR, false>(sp, w[k]);
         if (HIGH) any |= all;
     }
-    return any & 0x80808080u;
-}
-// Sweep filter of the long-buffer scan when the bytes that can FOLLOW a first byte are few (SET2): a unit passes only
-// if some byte of F's ranges is followed by one of (at most two) byte values, or by a lead byte if those can follow --
-// `^ERROR...`: (NUL | LF | CR) followed by `E` or LF.  That is the two-byte test of K2c for byte SETS; it cuts the
-// units that reach the confirm phase from "every line end" to "line ends in front of an E".
-template <int NR, bool HIGH>
-__device__ __forceinline__ uint32_t unit_any_set2(const SparseParams& sp, const uint4& a, const uint4& b) {
-    const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
-    uint32_t any = 0, z2_next = 0xFFFFFFFFu;
-#pragma unroll
-    for (int k = 7; k >= 0; k--) {
-        const uint32_t m1 = first_mask<NR, false>(sp, w[k]);
-        const uint32_t xa = w[k] ^ sp.second, xb = w[k] ^ sp.second_b;
-        const uint32_t z2 = ((xa - 0x01010101u) & ~xa) | ((xb - 0x01010101u) & ~xb) | (w[k] & sp.second_high);
-        any |= m1 & __funnelshift_r(z2, z2_next, 8);          // a first byte at j and a possible follower at j + 1
-        z2_next = z2;
-    }
-    if (HIGH) any |= w[0] | w[1] | w[2] | w[3] | w[4] | w[5] | w[6] | w[7];
     return any & 0x80808080u;
 }
 // bits 7, 15, 23, 31 of m -> bits 0..3
@@ -1208,12 +1183,13 @@ __device__ __noinline__ int sparse_run_units(const KParams& p, const SparseParam
     return sqn;                                                    // the start queue's new fill level
 }
 
-template <int KIND, int NR, bool HIGH, bool TWO, int MINB, int ROWS>
-__global__ void __launch_bounds__(256, MINB) k_in_sparse(KParams p, SparseParams sp, const uint8_t* __restrict__ buf,
-                                                      const int64_t* __restrict__ offsets, int64_t n, int64_t total,
-                                                      uint8_t* __restrict__ out, int spt, int64_t ntiles,
-                                                      int table_smem_bytes, int prezeroed, int flush_min, int stream_hint,
-                                                      int64_t stride) {
+// 4 CTAs per SM, 4 rows (4 KB per warp) in flight: the best of the measured combinations (DESIGN.md section 5)
+static constexpr int SPARSE_CTAS_PER_SM = 4, SPARSE_ROWS = 4;
+template <int KIND, int NR, bool HIGH, bool TWO>
+__global__ void __launch_bounds__(256, SPARSE_CTAS_PER_SM) k_in_sparse(KParams p, SparseParams sp, const uint8_t* __restrict__ buf,
+                                                                     const int64_t* __restrict__ offsets, int64_t n, int64_t total,
+                                                                     uint8_t* __restrict__ out, int spt, int64_t ntiles,
+                                                                     int table_smem_bytes, int prezeroed, int64_t stride) {
     extern __shared__ __align__(128) uint8_t smem[];
     uint8_t* s_cmap = smem;
     uint8_t* s_table = smem + 256;
@@ -1239,8 +1215,6 @@ __global__ void __launch_bounds__(256, MINB) k_in_sparse(KParams p, SparseParams
     const Anchored A{sp.flags, sp.start_nul, sp.q0};
     const uint32_t FULL = 0xffffffffu;
     const int nt = (int)ntiles;             // the host keeps n (hence ntiles) below 2^31
-    unsigned long long l2pol = 0;
-    if (stream_hint == 3) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(l2pol));
 
     // The warp's state machine.  The inner loop (no calls) advances it until 32 units or 32 starts are waiting or
     // the tiles are used up; the outer loop runs the queues and comes back.
@@ -1256,7 +1230,7 @@ __global__ void __launch_bounds__(256, MINB) k_in_sparse(KParams p, SparseParams
     int64_t nx0 = 0, nx1 = 0;               // byte range of the warp's next tile
     bool have_next = false;
 
-    bool drain = false;                     // run the queues even if they are not full (end of a tile, end of the tiles)
+    bool drain = false;                     // run the queues even if they are not full (the tiles are used up)
     for (;;) {
         for (;;) {
             if (uqn >= 32 || sqn >= 32 || drain) break;
@@ -1279,32 +1253,24 @@ __global__ void __launch_bounds__(256, MINB) k_in_sparse(KParams p, SparseParams
                 st = ST_SWEEP;
             }
             if (st == ST_SWEEP) {
-                // ---- S: up to 32 rows of 32 units, ROWS rows (ROWS KB per warp) in flight ----
+                // ---- S: up to 32 rows of 32 units, SPARSE_ROWS rows (SPARSE_ROWS KB per warp) in flight ----
                 const int64_t left = nunits - seg;
                 nrows = (int)((left < 1024 ? left : 1024) + 31) >> 5;
                 hitbits = 0;
                 uint32_t seen = 0;
-                for (int r = 0; r < nrows; r += ROWS) {
-                    uint4 va[ROWS], vb[ROWS];
+                for (int r = 0; r < nrows; r += SPARSE_ROWS) {
+                    uint4 va[SPARSE_ROWS], vb[SPARSE_ROWS];
 #pragma unroll
-                    for (int k = 0; k < ROWS; k++) {               // all loads first: ROWS KB per warp in flight
+                    for (int k = 0; k < SPARSE_ROWS; k++) {        // all loads first: SPARSE_ROWS KB per warp in flight
                         const int64_t u = seg + ((int64_t)(r + k) << 5) + lane;
                         va[k] = make_uint4(0, 0, 0, 0); vb[k] = va[k];
                         if (u < nunits && r + k < nrows) {
-                            if (stream_hint >= 2) {          // experiment: policies 2.. of ldg_v4_policy (L1 / L2 evict_last, ...)
-                                va[k] = ldg_v4_policy(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5)), stream_hint, l2pol);
-                                vb[k] = ldg_v4_policy(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5) + 16), stream_hint, l2pol);
-                            } else if (stream_hint) {
-                                va[k] = ldg_nc_v4(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5)));
-                                vb[k] = ldg_nc_v4(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5) + 16));
-                            } else {
-                                va[k] = __ldg(reinterpret_cast<const uint4*>(ubase + ((uintptr_t)u << 5)));
-                                vb[k] = __ldg(reinterpret_cast<const uint4*>(ubase + ((uintptr_t)u << 5) + 16));
-                            }
+                            va[k] = ldg_nc_v4(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5)));
+                            vb[k] = ldg_nc_v4(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5) + 16));
                         }
                     }
 #pragma unroll
-                    for (int k = 0; k < ROWS; k++) {
+                    for (int k = 0; k < SPARSE_ROWS; k++) {
                         const int64_t u = seg + ((int64_t)(r + k) << 5) + lane;
                         const uint32_t h = (u < nunits && r + k < nrows) ? unit_any<NR, HIGH, TWO>(sp, va[k], vb[k], seen) : 0u;
                         hitbits |= (h ? 1u : 0u) << (r + k);
@@ -1356,11 +1322,10 @@ __global__ void __launch_bounds__(256, MINB) k_in_sparse(KParams p, SparseParams
             seg += (int64_t)nrows << 5;
             if (seg < nunits) st = ST_SWEEP;
             else {
-                // Tile finished.  What it queued is still in L2 now -- a tile later it no longer is (the whole grid streams
-                // through L2 at once) -- so the queues are run here unless they hold next to nothing.
+                // Tile finished.  Its queued units and starts stay in the queues and are run with the next tile's once
+                // 32 are waiting; only after the warp's last tile are part-full queues drained.
                 st = ST_NEW;
                 t += gridDim.x * 8;
-                drain = flush_min > 0 && uqn + sqn >= flush_min;
             }
         }
         // ---- outer loop: run a queue (the only calls of the kernel) ----
@@ -1379,229 +1344,6 @@ __global__ void __launch_bounds__(256, MINB) k_in_sparse(KParams p, SparseParams
         } else {
             drain = false;                                         // both queues are empty
             if (st == ST_NEW && t >= nt) break;                    // ... and no tiles are left
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// K2p: K2 with length-balanced lanes.  A table lookup costs one shared-memory wavefront per warp instruction no
-// matter how many of the 32 lanes are still walking, so in K2 a warp whose strings are 64..256 bytes long wastes
-// a third of its lookups on lanes that have already finished.  Here a CTA of 128 threads takes a tile of up to
-// 256 strings, orders them by length (counting sort over 8-byte buckets, longest first) and gives thread j the
-// j-th longest and the j-th shortest string, one after the other: every lane then walks about the same number
-// of bytes and all warps of the CTA reach the tile barrier together.
-// ---------------------------------------------------------------------------------------------
-// layout: [0,16) mbarrier | classmap 256 | table | offsets (spt+4) x int32 | results spt | perm spt x u16 |
-//         hist 65 x int32 | pad to 128 | tile (cap+64)
-__host__ __device__ __forceinline__ int tile_offset_pairs(int table_smem_bytes, int spt) {
-    return (16 + 256 + table_smem_bytes + (spt + 4) * 4 + spt + spt * 2 + 65 * 4 + 127) & ~127;
-}
-
-template <int OP, int KIND>
-__global__ void __launch_bounds__(128, 8) k_bool_ragged_pairs(KParams p, const uint8_t* __restrict__ buf,
-                                                             const int64_t* __restrict__ offsets, int64_t n,
-                                                             int64_t total, uint8_t* __restrict__ out, int spt, int cap,
-                                                             int64_t ntiles, int table_smem_bytes) {
-    extern __shared__ __align__(128) uint8_t smem[];
-    uint8_t* s_cmap = smem + 16;
-    uint8_t* s_table = smem + 16 + 256;
-    int32_t* s_off = reinterpret_cast<int32_t*>(smem + 16 + 256 + table_smem_bytes);
-    uint8_t* s_res = reinterpret_cast<uint8_t*>(s_off + spt + 4);
-    uint16_t* s_perm = reinterpret_cast<uint16_t*>(s_res + spt);
-    int32_t* s_hist = reinterpret_cast<int32_t*>(s_perm + spt);
-    uint8_t* tile = smem + tile_offset_pairs(table_smem_bytes, spt);
-    const uint32_t mbar = smem_u32(smem);
-    Table<KIND> T = stage_table<KIND>(p, s_table, s_cmap);
-    if (threadIdx.x == 0) mbar_init(mbar, 1);
-    __syncthreads();
-    uint32_t phase = 0;
-    const uint32_t tile_addr = smem_u32(tile);
-    const int tid = threadIdx.x;
-    for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
-        const TileCtx c = load_tile(buf, offsets, n, total, t, spt, cap, tile, s_off, mbar, phase);
-        // ---- order by length: counting sort, 2 strings per thread (spt <= 256) ----
-        if (tid < 65) s_hist[tid] = 0;
-        __syncthreads();
-        int bucket[2], slot[2];
-#pragma unroll
-        for (int k = 0; k < 2; k++) {
-            const int i = tid + k * 128;
-            if (i < c.count) {
-                const int32_t r0 = s_off[i], r1 = s_off[i + 1];
-                const int len = r1 == OFF_BEYOND ? 0x7FFFFFF : r1 - r0;
-                int b = 63 - (len >> 3);
-                b = b < 0 ? 0 : b;
-                bucket[k] = b;
-                slot[k] = atomicAdd(&s_hist[b], 1);
-            }
-        }
-        __syncthreads();
-        if (tid < 32) {
-            const int a = s_hist[2 * tid], b2 = s_hist[2 * tid + 1];
-            const int sum = a + b2;
-            int inc = sum;
-            for (int d = 1; d < 32; d <<= 1) {
-                const int v = __shfl_up_sync(0xffffffffu, inc, d);
-                if (tid >= d) inc += v;
-            }
-            s_hist[2 * tid] = inc - sum;
-            s_hist[2 * tid + 1] = inc - sum + a;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int k = 0; k < 2; k++) {
-            const int i = tid + k * 128;
-            if (i < c.count) s_perm[s_hist[bucket[k]] + slot[k]] = (uint16_t)i;
-        }
-        __syncthreads();
-        // ---- thread j: the j-th longest, then the j-th shortest ----
-#pragma unroll
-        for (int k = 0; k < 2; k++) {
-            const int j = k == 0 ? tid : c.count - 1 - tid;
-            const bool mine = k == 0 ? (2 * tid < c.count + 0 && tid < c.count && tid <= c.count - 1 - tid)
-                                     : (c.count - 1 - tid > tid);
-            if (!mine) continue;
-            const int i = s_perm[j];
-            const int32_t r0 = s_off[i], r1 = s_off[i + 1];
-            bool r;
-            if (r1 == OFF_BEYOND) {
-                const int64_t o0 = __ldg(offsets + c.first + i), o1 = __ldg(offsets + c.first + i + 1);
-                r = eval_bool_slow<OP>(p, buf + o0, o1 - o0);
-            } else {
-                const int len = r1 - r0;
-                const uint32_t a = tile_addr + (uint32_t)r0;
-                if (degenerate_text<OP>(len, len ? lds_u8(a) : 0)) r = p.q0_accepting != 0;
-                else {
-                    uint32_t high = 0;
-                    r = result_flag(p, walk_smem(T, (uint32_t)p.start, a, len, high));
-                    if (OP == 1 && r && p.prefix_mode == 1 && (high & 0x80808080u))
-                        r = recheck_in_with_prefix(p, buf + (c.base + r0), len);
-                }
-            }
-            s_res[i] = r ? 1 : 0;
-        }
-        __syncthreads();
-        for (int i = tid; i < c.count; i += 128) out[c.first + i] = s_res[i];
-        __syncthreads();
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// K2s: ragged batch, boolean result, streaming form.
-// The flat buffer is cut into windows of `window` bytes; a thread owns the strings that START inside its
-// window and streams through them in address order (they are contiguous), reading the text straight from
-// global memory as aligned 16-byte loads with the next chunk always in flight.  A string boundary is just
-// "record the result, reset the state".  Compared with the tile form there is no shared-memory text (shared
-// memory only holds the table, so text reads cost no bank conflicts), no block barrier, and a thread's work
-// is its window plus/minus one string, which keeps the 32 lanes of a warp busy regardless of how ragged the
-// strings are.  Consecutive lanes own consecutive windows, so a warp sweeps one contiguous region.
-// ---------------------------------------------------------------------------------------------
-struct StreamCold {   // per-thread bookkeeping that only the (rare, out-of-line) string-boundary code touches
-    int64_t s;        // current string
-    int64_t o0;       // its start
-    int64_t o2;       // offsets[s + 2], prefetched
-};
-
-// The current string [C.o0, o1) ends after the byte just consumed (b): write its result and move to the next
-// string that starts inside the window (empty strings in between are answered on the spot).  Returns the end
-// offset of the new current string, or -1 when the thread's window is exhausted.
-template <int OP>
-__device__ __noinline__ int64_t stream_emit(const KParams& p, const uint8_t* __restrict__ buf,
-                                            const int64_t* __restrict__ offsets, int64_t n, int64_t w1,
-                                            uint8_t* __restrict__ out, StreamCold& C, int64_t o1, uint32_t st,
-                                            uint32_t b, uint32_t high) {
-    bool r = result_flag(p, st);
-    const int64_t len = o1 - C.o0;
-    if (OP == 1 && len == 1 && b == 0x20) r = p.q0_accepting != 0;     // single blank: api_internal_m.F90:68-74
-    if (OP == 1 && r && p.prefix_mode == 1 && (high & 0x80808080u)) r = recheck_in_with_prefix(p, buf + C.o0, len);
-    out[C.s] = r ? 1 : 0;
-    C.s++;
-    C.o0 = o1;
-    o1 = C.o2;
-    while (C.s < n && C.o0 < w1 && o1 == C.o0) {                       // empty strings
-        out[C.s] = p.q0_accepting ? 1 : 0;
-        C.s++;
-        o1 = C.s + 1 <= n ? __ldg(offsets + C.s + 1) : o1;
-    }
-    if (C.s >= n || C.o0 >= w1) return -1;
-    C.o2 = C.s + 2 <= n ? __ldg(offsets + C.s + 2) : o1;
-    return o1;
-}
-
-template <int OP, int KIND>
-__global__ void __launch_bounds__(256, 4) k_bool_stream(KParams p, const uint8_t* __restrict__ buf,
-                                                        const int64_t* __restrict__ offsets, int64_t n, int64_t total,
-                                                        uint8_t* __restrict__ out, int window, int64_t nwindows) {
-    extern __shared__ __align__(128) uint8_t smem[];
-    uint8_t* s_cmap = smem;
-    uint8_t* s_table = smem + 256;
-    Table<KIND> T = stage_table<KIND>(p, s_table, s_cmap);
-    if (KIND != 3) __syncthreads();
-    const uintptr_t gbuf = reinterpret_cast<uintptr_t>(buf);
-    const uintptr_t glast = (gbuf + (uintptr_t)total + 15) & ~(uintptr_t)15;   // end of the last 16-byte block that holds text
-    const uint32_t start = (uint32_t)p.start;
-    for (int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; w < nwindows;
-         w += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t w0 = w * window;
-        const int64_t w1 = (w == nwindows - 1) ? total + 1 : w0 + window;   // strings with o0 in [w0, w1)
-        StreamCold C;
-        {   // first string that starts at or after w0
-            int64_t lo = 0, hi = n;
-            while (lo < hi) {
-                const int64_t mid = (lo + hi) >> 1;
-                if (__ldg(offsets + mid) < w0) lo = mid + 1; else hi = mid;
-            }
-            C.s = lo;
-        }
-        if (C.s >= n) continue;
-        C.o0 = __ldg(offsets + C.s);
-        if (C.o0 >= w1) continue;
-        int64_t o1 = __ldg(offsets + C.s + 1);
-        bool done = false;
-        while (o1 == C.o0) {                                             // leading empty strings
-            out[C.s] = p.q0_accepting ? 1 : 0;
-            C.s++;
-            if (C.s >= n) { done = true; break; }
-            o1 = __ldg(offsets + C.s + 1);
-        }
-        if (done) continue;
-        C.o2 = C.s + 2 <= n ? __ldg(offsets + C.s + 2) : o1;
-        uint32_t st = start;
-        // the thread's private stream: aligned 16-byte chunks; (cp, k0) = next unread byte
-        const uint4* cp = reinterpret_cast<const uint4*>((gbuf + (uintptr_t)C.o0) & ~(uintptr_t)15);
-        int k0 = (int)((gbuf + (uintptr_t)C.o0) & 15);
-        int64_t cbase = C.o0 - k0;                                       // buffer offset of the chunk's first byte
-        uint4 cur = __ldg(cp);
-        uint4 nxt = make_uint4(0, 0, 0, 0);
-        if (reinterpret_cast<uintptr_t>(cp + 1) < glast) nxt = __ldg(cp + 1);
-        uint32_t high = 0;
-        while (true) {
-            const uint32_t wv[4] = {cur.x, cur.y, cur.z, cur.w};
-            const uint32_t chigh = cur.x | cur.y | cur.z | cur.w;
-            high |= chigh;
-            const int64_t rem64 = o1 - (cbase + k0);                        // bytes until the current string ends (>= 1)
-            const int kend = rem64 < (int64_t)(16 - k0) ? k0 + (int)rem64 : 16;
-            const uint32_t mask = (0xFFFFu >> (16 - kend)) & (0xFFFFu << k0);
-#pragma unroll
-            for (int k = 0; k < 16; k++) {
-                if (mask & (1u << k)) st = T.next(st, (wv[k >> 2] >> (8 * (k & 3))) & 0xFF);
-            }
-            if ((int64_t)(kend - k0) == rem64) {                            // the string ended inside this chunk
-                const uint32_t b = (wv[(kend - 1) >> 2] >> (8 * ((kend - 1) & 3))) & 0xFF;
-                o1 = stream_emit<OP>(p, buf, offsets, n, w1, out, C, o1, st, b, high);
-                if (o1 < 0) break;
-                st = start;
-                high = chigh;
-            }
-            if (kend == 16) {                                               // move to the next chunk, keep one in flight
-                cp++;
-                cbase += 16;
-                k0 = 0;
-                cur = nxt;
-                if (reinterpret_cast<uintptr_t>(cp + 1) < glast) nxt = __ldg(cp + 1);
-            } else {
-                k0 = kend;
-            }
         }
     }
 }
@@ -1839,11 +1581,11 @@ __host__ __device__ __forceinline__ SpanHead span_head(int fwd_bytes, int rdelta
 }
 static constexpr int SPAN_ROUND = 64;            // bytes a lane walks before the warp looks for idle lanes again (C3: 16 -> 701, 32 -> 777, 64 -> 816 GB/s)
 
-template <int FK, bool RS, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, 1) k_span_ragged(KParams p, SpanParams sp, const uint8_t* __restrict__ buf,
-                                                                   const int64_t* __restrict__ offsets, int64_t n, int64_t total,
-                                                                   int64_t* __restrict__ from, int64_t* __restrict__ to,
-                                                                   int spt, int cap, int64_t ntiles, int fwd_bytes, int round_bytes) {
+template <int FK, bool RS>
+__global__ void __launch_bounds__(SPAN_WARPS * 32, 1) k_span_ragged(KParams p, SpanParams sp, const uint8_t* __restrict__ buf,
+                                                                        const int64_t* __restrict__ offsets, int64_t n, int64_t total,
+                                                                        int64_t* __restrict__ from, int64_t* __restrict__ to,
+                                                                        int spt, int cap, int64_t ntiles, int fwd_bytes) {
     extern __shared__ __align__(128) uint8_t smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t FULL = 0xffffffffu;
@@ -1887,8 +1629,8 @@ __global__ void __launch_bounds__(WARPS * 32, 1) k_span_ragged(KParams p, SpanPa
     uint32_t phase = 0;
     const uint32_t tile_addr = smem_u32(tile);
     const uintptr_t gbuf = reinterpret_cast<uintptr_t>(buf);
-    const int64_t nwarps = (int64_t)gridDim.x * WARPS;
-    for (int64_t t = (int64_t)blockIdx.x * WARPS + warp; t < ntiles; t += nwarps) {
+    const int64_t nwarps = (int64_t)gridDim.x * SPAN_WARPS;
+    for (int64_t t = (int64_t)blockIdx.x * SPAN_WARPS + warp; t < ntiles; t += nwarps) {
         // ---- stage the tile: strings [first, first + count), up to `cap` bytes of them ----
         const int64_t first = t * spt;
         const int count = (int)((n - first) < spt ? (n - first) : spt);
@@ -1981,7 +1723,7 @@ __global__ void __launch_bounds__(WARPS * 32, 1) k_span_ragged(KParams p, SpanPa
             }
             if (!__any_sync(FULL, have)) { if (next >= count) break; else continue; }
             if (have) {
-                int jend = (int)(((a + (uint32_t)j + (uint32_t)round_bytes) & ~3u) - a);     // the round ends on a word boundary of the tile
+                int jend = (int)(((a + (uint32_t)j + SPAN_ROUND) & ~3u) - a);     // the round ends on a word boundary of the tile
                 if (jend > len) jend = len;
                 while (j < jend && ((a + (uint32_t)j) & 3u)) { const uint32_t b = lds_u8(a + j); FX_SPAN_STEP(T, st, last, b, j); j++; }
                 for (; j + 4 <= jend && st != 0; j += 4) {
@@ -2032,274 +1774,6 @@ __global__ void __launch_bounds__(WARPS * 32, 1) k_span_ragged(KParams p, SpanPa
 }
 
 // ---------------------------------------------------------------------------------------------
-// K3f, streaming form (EXPERIMENT, FX_SPAN_STREAM=1; not the default: 403 vs 720 GB/s on C3 -- the walker state needs
-// ~110 registers, so 16 warps per SM instead of 32, and the busy-lane count per instruction did not move (14.8 of 32
-// either way: the idle lanes of K3f sit INSIDE the walks -- rounds cut short by a dying state, byte-wise heads and tails,
-// the divergent backward decode -- not between strings).  Same walks as k_span_ragged above; what changes is that a warp never waits for a
-// tile to finish.  Every warp owns a RING of NB small buffers (its share of shared memory cut in NB pieces, each filled
-// by its own TMA bulk copy on its own mbarrier).  The 32 lanes are walkers: a lane without a string claims the next
-// unclaimed string of the oldest buffer that has one -- no matter whether the other lanes are still busy with earlier
-// strings -- and walks it 32 bytes per round.  A buffer is flushed (results written as one coalesced run) and refilled
-// with the warp's next tile as soon as its last string is complete, while the lanes are already at work in the next
-// buffer.  A forward walk that ends with a match leaves a backward JOB in the lane (the lane goes on claiming); the
-// jobs of the warp are run together when 16 lanes hold one, when a lane would need a second slot, or when nothing else
-// is left to do -- so both walks run with most lanes busy.
-// With per-tile passes (above) a warp walked ~2 strings per lane and then waited for its slowest lane, and ran its
-// backward walks in half-empty batches: 46 % of the lanes were busy on C3.
-// ---------------------------------------------------------------------------------------------
-static constexpr int RING_NB = 3;
-struct RingLayout { int off_res, off_text, buf_bytes; };
-__host__ __device__ __forceinline__ RingLayout ring_layout(int spt, int cap) {
-    RingLayout L;
-    L.off_res = (16 + (spt + 4) * 4 + 7) & ~7;
-    L.off_text = (L.off_res + spt * 8 + 127) & ~127;
-    L.buf_bytes = (L.off_text + cap + 64 + 127) & ~127;
-    return L;
-}
-
-template <int FK, bool RS, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, 1) k_span_stream(KParams p, SpanParams sp, const uint8_t* __restrict__ buf,
-                                                              const int64_t* __restrict__ offsets, int64_t n, int64_t total,
-                                                              int64_t* __restrict__ from, int64_t* __restrict__ to,
-                                                              int spt, int cap, int64_t ntiles, int fwd_bytes) {
-    extern __shared__ __align__(128) uint8_t smem[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t FULL = 0xffffffffu;
-    const SpanHead H = span_head(fwd_bytes, sp.rstates * sp.rclasses * 2, sp.nmixed, RS);
-    const RingLayout L = ring_layout(spt, cap);
-    // ---- stage the tables (the only block-wide step) ----
-    SpanFwd<FK> T;
-    T.s_cmap = smem_u32(smem); T.s_table = smem_u32(smem + 256); T.g_table = sp.table; T.g_cmap = sp.classmap; T.shift = sp.row_shift;
-    if (FK == 0) {
-        uint16_t* dst = reinterpret_cast<uint16_t*>(smem + 256);
-        for (int i = threadIdx.x; i < sp.nstates * 128; i += blockDim.x) {
-            const uint32_t v = __ldg(reinterpret_cast<const uint32_t*>(sp.direct) + i);
-            *reinterpret_cast<uint32_t*>(dst + (i >> 7) * SPAN_ROW + ((i & 127) << 1)) = v;
-        }
-    } else if (FK == 1) {
-        uint32_t* dst = reinterpret_cast<uint32_t*>(smem + 256);
-        const int words32 = ((sp.nstates << sp.row_shift) + 1) >> 1;
-        for (int i = threadIdx.x; i < words32; i += blockDim.x) dst[i] = __ldg(reinterpret_cast<const uint32_t*>(sp.table) + i);
-        for (int i = threadIdx.x; i < 64; i += blockDim.x)
-            reinterpret_cast<uint32_t*>(smem)[i] = __ldg(reinterpret_cast<const uint32_t*>(sp.classmap) + i);
-    }
-    SpanRev<RS> R;
-    R.s_delta = smem_u32(smem + H.off_rdelta); R.s_page = smem_u32(smem + H.off_page); R.s_mixed = smem_u32(smem + H.off_mixed);
-    if (RS) {
-        uint16_t* d = reinterpret_cast<uint16_t*>(smem + H.off_rdelta);
-        for (int i = threadIdx.x; i < sp.rstates * sp.rclasses; i += blockDim.x) d[i] = __ldg(sp.rdelta + i);
-        for (int i = threadIdx.x; i < 1024; i += blockDim.x) smem[H.off_page + i] = __ldg(sp.rpage + i);
-        for (int i = threadIdx.x; i < sp.nmixed * 64; i += blockDim.x) smem[H.off_mixed + i] = __ldg(sp.rmixed + i);
-    }
-    uint8_t* ring = smem + H.bytes + warp * (RING_NB * L.buf_bytes);
-    if (lane < RING_NB) mbar_init(smem_u32(ring + lane * L.buf_bytes), 1);
-    __syncthreads();
-    const uintptr_t gbuf = reinterpret_cast<uintptr_t>(buf);
-    const int64_t nwarps = (int64_t)gridDim.x * WARPS;
-    int64_t next_tile = (int64_t)blockIdx.x * WARPS + warp;          // the warp's tiles: next_tile, next_tile + nwarps, ...
-
-    // ring bookkeeping (warp-uniform): per buffer the tile it holds, how many strings, how many claimed / complete
-    int64_t b_first[RING_NB];
-    int b_count[RING_NB], b_claimed[RING_NB], b_done[RING_NB];
-    uint32_t b_phase[RING_NB];
-    bool b_loaded[RING_NB], b_ready[RING_NB];
-#pragma unroll
-    for (int x = 0; x < RING_NB; x++) { b_first[x] = 0; b_count[x] = 0; b_claimed[x] = 0; b_done[x] = 0; b_phase[x] = 0; b_loaded[x] = false; b_ready[x] = false; }
-    int oldest = 0;                                                   // claims go through the buffers in ring order from here
-
-    // lane state: the forward walk in hand, and one backward job
-    bool have = false;
-    int f_buf = 0, f_sidx = 0, f_len = 0, j = 0, last = -1;
-    uint32_t f_a = 0, st = 0;
-    bool job = false, spill = false;                                  // spill: a finished forward walk waits for the job slot
-    int j_buf = 0, j_sidx = 0, j_len = 0, j_last = 0;
-    uint32_t j_a = 0;
-
-    for (;;) {
-        // ---- 1. flush complete buffers, load the warp's next tiles into free ones ----
-#pragma unroll
-        for (int x = 0; x < RING_NB; x++) {
-            if (b_loaded[x] && b_done[x] == b_count[x]) {
-                const int2* s_res = reinterpret_cast<const int2*>(ring + x * L.buf_bytes + L.off_res);
-                __syncwarp();
-                for (int i = lane; i < b_count[x]; i += 32) {
-                    const int2 r = s_res[i];
-                    if (r.x >= 0) { from[b_first[x] + i] = r.x; to[b_first[x] + i] = r.y; }
-                }
-                b_loaded[x] = false;
-                __syncwarp();
-            }
-            if (!b_loaded[x] && next_tile < ntiles) {
-                uint8_t* B = ring + x * L.buf_bytes;
-                int32_t* s_off = reinterpret_cast<int32_t*>(B + 16);
-                uint8_t* text = B + L.off_text;
-                const int64_t first = next_tile * spt;
-                const int count = (int)((n - first) < spt ? (n - first) : spt);
-                const int64_t t0 = __ldg(offsets + first), tend = __ldg(offsets + first + count);
-                const int64_t t1 = tend - t0 > cap ? t0 + cap : tend;
-                const uintptr_t g0 = gbuf + (uintptr_t)t0;
-                const int64_t base = t0 - (int64_t)(g0 & 15);
-                const uintptr_t gsrc = g0 & ~(uintptr_t)15;
-                uintptr_t gcopy_end = (gbuf + (uintptr_t)t1 + 15) & ~(uintptr_t)15;
-                const uintptr_t gsafe_end = (gbuf + (uintptr_t)total) & ~(uintptr_t)15;
-                if (gcopy_end > gsafe_end) gcopy_end = gsafe_end;
-                const uint32_t bulk = gcopy_end > gsrc ? (uint32_t)(gcopy_end - gsrc) : 0u;
-                if (lane == 0) {
-                    const uint32_t mbar = smem_u32(B);
-                    mbar_expect_tx(mbar, bulk);
-                    if (bulk) bulk_g2s(smem_u32(text), reinterpret_cast<const void*>(gsrc), bulk, mbar);
-                }
-                for (int64_t xx = (int64_t)(gsrc + bulk) - (int64_t)gbuf + lane; xx < t1; xx += 32)
-                    if (xx >= t0) text[xx - base] = __ldg(buf + xx);
-                for (int i = lane; i <= count; i += 32) {
-                    const int64_t o = __ldg(offsets + first + i);
-                    s_off[i] = o > t1 ? OFF_BEYOND : (int32_t)(o - base);
-                }
-                b_first[x] = first; b_count[x] = count; b_claimed[x] = 0; b_done[x] = 0;
-                b_loaded[x] = true; b_ready[x] = false;
-                next_tile += nwarps;
-                __syncwarp();
-            }
-        }
-        // ---- 2. idle lanes claim strings, oldest buffer first ----
-        uint32_t idle = __ballot_sync(FULL, !have && !spill);
-        bool starving = false;
-#pragma unroll
-        for (int k = 0; k < RING_NB; k++) {
-            const int x = (oldest + k) % RING_NB;
-            bool usable = false;
-            int cl = 0, cnt = 0;
-#pragma unroll
-            for (int y = 0; y < RING_NB; y++) if (y == x) { usable = b_loaded[y] && b_claimed[y] < b_count[y]; cl = b_claimed[y]; cnt = b_count[y]; }
-            if (idle == 0 || !usable) continue;
-            bool ready = false;
-#pragma unroll
-            for (int y = 0; y < RING_NB; y++) if (y == x) ready = b_ready[y];
-            if (!ready) {
-                // the copy may still be in flight: wait for it only if no lane has anything else to do
-                const bool busy = __any_sync(FULL, have || job);
-                uint32_t ph = 0;
-#pragma unroll
-                for (int y = 0; y < RING_NB; y++) if (y == x) ph = b_phase[y];
-                uint32_t ok = 0;
-                const uint32_t mbar = smem_u32(ring + x * L.buf_bytes);
-                if (busy) {
-                    asm volatile("{ .reg .pred p; mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                                 : "=r"(ok) : "r"(mbar), "r"(ph) : "memory");
-                    ok = __all_sync(FULL, ok != 0) ? 1u : 0u;
-                } else { mbar_wait(mbar, ph); ok = 1; }
-                if (!ok) { starving = true; break; }                 // (older strings first: do not skip ahead of a buffer in flight)
-#pragma unroll
-                for (int y = 0; y < RING_NB; y++) if (y == x) { b_ready[y] = true; b_phase[y] ^= 1; }
-                __syncwarp();
-            }
-            const int32_t* s_off = reinterpret_cast<const int32_t*>(ring + x * L.buf_bytes + 16);
-            int2* s_res = reinterpret_cast<int2*>(ring + x * L.buf_bytes + L.off_res);
-            const uint32_t text_addr = smem_u32(ring + x * L.buf_bytes + L.off_text);
-            const int mine = cl + __popc(idle & ((1u << lane) - 1));
-            int finished_here = 0;                                   // strings decided at claim time
-            bool took = false;
-            if (((idle >> lane) & 1u) && mine < cnt) {
-                took = true;
-                const int32_t r0 = s_off[mine], r1 = s_off[mine + 1];
-                int64_t bf = 0;
-#pragma unroll
-                for (int y = 0; y < RING_NB; y++) if (y == x) bf = b_first[y];
-                if (r1 == OFF_BEYOND) {          // longer than a buffer: the same two walks, text from global memory
-                    const int64_t o0 = __ldg(offsets + bf + mine), o1 = __ldg(offsets + bf + mine + 1);
-                    int64_t f = 0, e = 0;
-                    if (o1 - o0 == 0 || (o1 - o0 == 1 && __ldg(buf + o0) == 0x20)) {
-                    } else if (o1 - o0 < 0x7FFFFFF0ll) {
-                        span_linear(sp, T, R, FetchGlobal{buf + o0}, (int)(o1 - o0), f, e);
-                    } else {
-                        Table<3> G;
-                        G.g_table = p.ctable; G.g_cmap = p.classmap; G.shift = p.c_row_shift; G.s_table = 0; G.s_cmap = 0;
-                        eval_regex(p, G, FetchGlobal{buf + o0}, o1 - o0, f, e);
-                    }
-                    from[bf + mine] = f; to[bf + mine] = e;
-                    s_res[mine] = make_int2(-1, -1);
-                    finished_here = 1;
-                } else {
-                    f_len = r1 - r0;
-                    f_a = text_addr + (uint32_t)r0;
-                    if (f_len == 0 || (f_len == 1 && lds_u8(f_a) == 0x20)) { s_res[mine] = make_int2(0, 0); finished_here = 1; }   // api_internal_m.F90:68-74
-                    else { have = true; f_buf = x; f_sidx = mine; j = 0; st = (uint32_t)sp.start; last = sp.start_acc ? 0 : -1; }
-                }
-            }
-            const int ntook = __popc(__ballot_sync(FULL, took));
-            const int nfin = __popc(__ballot_sync(FULL, finished_here != 0));
-#pragma unroll
-            for (int y = 0; y < RING_NB; y++) if (y == x) { b_claimed[y] += ntook; b_done[y] += nfin; }
-            idle = __ballot_sync(FULL, !have && !spill && !took);    // (a lane that took a degenerate string may claim again next round)
-        }
-        // the oldest buffer moves on once every string of it is claimed
-#pragma unroll
-        for (int k = 0; k < RING_NB; k++) {
-            bool exhausted = false;
-#pragma unroll
-            for (int y = 0; y < RING_NB; y++) if (y == oldest) exhausted = !b_loaded[y] || b_claimed[y] >= b_count[y];
-            bool any_other = false;
-#pragma unroll
-            for (int y = 0; y < RING_NB; y++) if (y != oldest && b_loaded[y] && b_claimed[y] < b_count[y]) any_other = true;
-            if (exhausted && any_other) oldest = (oldest + 1) % RING_NB; else break;
-        }
-        // ---- 3. one round of forward walking ----
-        int fin_buf = -1;                                            // this lane completed a string of buffer fin_buf without a match
-        if (have) {
-            int jend = (int)(((f_a + (uint32_t)j + SPAN_ROUND) & ~3u) - f_a);
-            if (jend > f_len) jend = f_len;
-            while (j < jend && ((f_a + (uint32_t)j) & 3u)) { const uint32_t bb = lds_u8(f_a + j); FX_SPAN_STEP(T, st, last, bb, j); j++; }
-            for (; j + 4 <= jend && st != 0; j += 4) {
-                const uint32_t w4 = lds_u32(f_a + j);
-                const uint32_t n1 = T.next(st, w4 & 0xFFu);
-                const uint32_t n2 = T.next(n1 & W_SSTATE, (w4 >> 8) & 0xFFu);
-                const uint32_t n3 = T.next(n2 & W_SSTATE, (w4 >> 16) & 0xFFu);
-                const uint32_t n4 = T.next(n3 & W_SSTATE, w4 >> 24);
-                if ((n1 | n2 | n3 | n4) & 0xB000u) {
-                    FX_SPAN_BOOKS4(n1, n2, n3, n4, last, j);
-                }
-                st = n4 & W_SSTATE;
-            }
-            if (st != 0) for (; j < jend; j++) { const uint32_t bb = lds_u8(f_a + j); FX_SPAN_STEP(T, st, last, bb, j); }
-            if (st == 0 || j >= f_len) {
-                if (st != 0) last = span_end_of_text(sp, st, f_len, last);
-                have = false;
-                if (last <= 0) {                                     // no match, or only the leading NUL matched (to = 0)
-                    reinterpret_cast<int2*>(ring + f_buf * L.buf_bytes + L.off_res)[f_sidx] = make_int2(0, 0);
-                    fin_buf = f_buf;
-                } else if (!job) { job = true; j_buf = f_buf; j_sidx = f_sidx; j_len = f_len; j_last = last; j_a = f_a; }
-                else spill = true;                                   // the job slot is taken: the warp runs its jobs now
-            }
-        }
-#pragma unroll
-        for (int y = 0; y < RING_NB; y++) b_done[y] += __popc(__ballot_sync(FULL, fin_buf == y));
-        // ---- 4. backward jobs: when half the lanes hold one, when a lane needs the slot, or when nothing else is left ----
-        const uint32_t jobs = __ballot_sync(FULL, job);
-        const bool any_spill = __any_sync(FULL, spill);
-        const bool any_fwd = __any_sync(FULL, have);
-        (void)starving;
-        if (jobs != 0 && (__popc(jobs) >= 16 || any_spill || !any_fwd)) {      // (!any_fwd: no lane found a string to walk this round)
-            int jb = -1;
-            if (job) {
-                const int f = span_backward(sp, R, FetchShared{j_a}, j_len, j_last);
-                reinterpret_cast<int2*>(ring + j_buf * L.buf_bytes + L.off_res)[j_sidx] =
-                    f > 0 ? make_int2(f, j_last < j_len ? j_last : j_len) : make_int2(0, 0);
-                jb = j_buf;
-                job = false;
-            }
-            if (spill) { job = true; spill = false; j_buf = f_buf; j_sidx = f_sidx; j_len = f_len; j_last = last; j_a = f_a; }
-#pragma unroll
-            for (int y = 0; y < RING_NB; y++) b_done[y] += __popc(__ballot_sync(FULL, jb == y));
-        }
-        // ---- 5. done? ----
-        bool pending = __any_sync(FULL, have || job || spill) || next_tile < ntiles;
-#pragma unroll
-        for (int y = 0; y < RING_NB; y++) if (b_loaded[y]) pending = true;
-        if (!pending) break;
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
 // K4: one long buffer, span result (config C4).
 // The reference tries every character boundary as a start, in order, and returns at the first one
 // whose anchored run accepts after >= 1 symbol (api_internal_m.F90:108-155).  The attempts are
@@ -2338,7 +1812,6 @@ struct ScanBudget {
     unsigned long long* work;    // steps so far (all warps)
     unsigned long long* abort;   // set once the budget is spent
     unsigned long long limit;
-    int flags;                   // experiments (FX_K4_FLAGS): 1 = no prefetch in front of an attempt, 2 = the plain loop without budget chunks
 };
 static constexpr int BUDGET_TICK = 65536;        // steps a lane walks between two looks at the shared counter (one atomic each:
                                                  // at 4096 the 420 K same-address atomics of C4's attempts cost 3 ms of its 15)
@@ -2431,7 +1904,7 @@ __global__ void __launch_bounds__(256) k_buffer_scan(KParams p, const uint8_t* _
                                                      const unsigned long long* __restrict__ run_if) {
     if (gate != nullptr && *gate != 0) return;      // the prefix occurs in the text: its occurrences were the candidates
     if (run_if != nullptr && *run_if == 0) return;  // fallback behind the state-map scan: only if that scan declined
-    const ScanBudget B{nullptr, nullptr, 0ull, 0};
+    const ScanBudget B{nullptr, nullptr, 0ull};
     uint32_t acc = 0;
     extern __shared__ __align__(128) uint8_t smem[];
     uint8_t* s_cmap = smem;
@@ -2575,11 +2048,11 @@ __host__ __device__ __forceinline__ int scan_sparse_smem_bytes(int table_smem_by
 // the literal's first byte, the unit phase compares the whole literal, and best[2] counts the occurrences seen: when
 // the literal occurs nowhere the reference falls back to all boundaries -- the caller then runs the plain scan, which
 // is gated on best[2] == 0.  The start on the leading NUL is tried iff the literal sits at the very front of the text.
-template <int KIND, int NR, bool HIGH, bool PREFIX, bool SET2>
+template <int KIND, int NR, bool HIGH, bool PREFIX>
 __global__ void __launch_bounds__(256) k_buffer_scan_sparse(KParams p, SparseParams sp, const uint8_t* __restrict__ buf,
                                                             ScanWindow W, unsigned long long* __restrict__ best,
                                                             int table_smem_bytes, const unsigned long long* __restrict__ gate,
-                                                            int phases, const unsigned long long* __restrict__ run_if, ScanBudget B) {
+                                                            const unsigned long long* __restrict__ run_if, ScanBudget B) {
     if (gate != nullptr && *gate != 0) return;      // (plain scan of a prefix pattern) the prefix occurs in the text
     if (run_if != nullptr && *run_if == 0) return;  // fallback behind the state-map scan: only if that scan declined
     uint32_t acc = 0;
@@ -2622,7 +2095,7 @@ __global__ void __launch_bounds__(256) k_buffer_scan_sparse(KParams p, SparsePar
             if (lane == 0) ab = *reinterpret_cast<volatile unsigned long long*>(B.abort);
             if (__shfl_sync(FULL, ab, 0) != 0) return;
         }
-        if (lane < count && (phases & 2)) {
+        if (lane < count) {
             const int64_t pos = s_starts[lane];
             if (try_start(p, T, buf, len, pos, __ldg(buf + pos), open_end, overflow, B, acc))
                 atomicMin(best, (unsigned long long)(W.origin + pos) + 2);
@@ -2633,7 +2106,7 @@ __global__ void __launch_bounds__(256) k_buffer_scan_sparse(KParams p, SparsePar
         __syncwarp();
         uint32_t cand = 0;
         int64_t P = 0;
-        if (lane < count && (phases & 1)) {
+        if (lane < count) {
             const int64_t u = s_units[lane];
             const uintptr_t ua = ubase + ((uintptr_t)u << 5);
             const uint4 v0 = __ldg(reinterpret_cast<const uint4*>(ua)), v1 = __ldg(reinterpret_cast<const uint4*>(ua + 16));
@@ -2641,21 +2114,6 @@ __global__ void __launch_bounds__(256) k_buffer_scan_sparse(KParams p, SparsePar
                    (pack_byte_flags(first_mask<NR, HIGH>(sp, v0.z)) << 8) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v0.w)) << 12) |
                    (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.x)) << 16) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.y)) << 20) |
                    (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.z)) << 24) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.w)) << 28);
-            if (SET2) {
-                // two-byte test: a candidate whose follower is none of the (at most two) byte values that can follow a
-                // first byte -- nor a lead byte, if those can -- is dead.  The follower of the unit's last byte is not
-                // here: that candidate stays.  (Lead bytes >= 0xC0 as FIRST bytes enter a sequence: they stay as well.)
-                const uint32_t w8[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
-                uint32_t fol = 0, lead = 0;
-#pragma unroll
-                for (int q = 0; q < 8; q++) {
-                    const uint32_t xa = w8[q] ^ sp.second, xb = w8[q] ^ sp.second_b;
-                    const uint32_t z2 = ((xa - 0x01010101u) & ~xa) | ((xb - 0x01010101u) & ~xb) | (w8[q] & sp.second_high);
-                    fol |= pack_byte_flags(z2) << (4 * q);
-                    lead |= pack_byte_flags(w8[q]) << (4 * q);
-                }
-                cand &= (fol >> 1) | 0x80000000u | lead;
-            }
             P = pos_base + (u << 5);
             if (P < W.start_lo) cand &= 0xFFFFFFFFu << (int)(W.start_lo - P);
             if (P + 32 > W.start_hi) cand &= (P >= W.start_hi) ? 0u : (0xFFFFFFFFu >> (int)(P + 32 - W.start_hi));
@@ -2703,9 +2161,6 @@ __global__ void __launch_bounds__(256) k_buffer_scan_sparse(KParams p, SparsePar
 
     const int64_t gwarp = (int64_t)blockIdx.x * 8 + warp, nwarps = (int64_t)gridDim.x * 8;
     int sweep_iter = 0;
-    const int lp = (phases >> 4) & 7;
-    unsigned long long l2pol = 0;
-    if (lp == 3) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(l2pol));
     for (int64_t g0 = gwarp * 128; g0 < nunits; g0 += nwarps * 128) {
         unsigned long long cur = 0;
         if (lane == 0) cur = *reinterpret_cast<volatile unsigned long long*>(best);
@@ -2722,8 +2177,8 @@ __global__ void __launch_bounds__(256) k_buffer_scan_sparse(KParams p, SparsePar
             const int64_t u = g0 + k * 32 + lane;
             va[k] = make_uint4(0, 0, 0, 0); vb[k] = va[k];
             if (u < nunits) {
-                va[k] = ldg_v4_policy(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5)), lp, l2pol);
-                vb[k] = ldg_v4_policy(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5) + 16), lp, l2pol);
+                va[k] = ldg_v4(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5)));
+                vb[k] = ldg_v4(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5) + 16));
             }
         }
 #pragma unroll

@@ -268,7 +268,7 @@ def test_c5_in_fixed_big_table(residency, compact, monkeypatch):
 
 
 # ---- edge cases: empty / ragged / long / unaligned -------------------------------------------------
-def test_ragged_edge_cases():
+def test_ragged_edge_cases(monkeypatch):
     rng = np.random.default_rng(7)
     strings = [b"", b" ", b"a", b"", b"", b"foobar", b"x" * 5000 + b"foobaz", b"y" * 70000, b"foobar" * 3, b"",
                bytes(rng.integers(0, 256, size=300, dtype=np.uint8)), b"\x00", b"\xe3\x81", b"fooba", b""]
@@ -282,6 +282,24 @@ def test_ragged_edge_cases():
         got = p.in_batch(buf, off) if op == "in" else p.match_batch(buf, off)
         exp = oracle_bool(pat, op, buf, offsets=off)
         assert np.array_equal(got, exp), (pat, op, np.nonzero(got != exp)[0][:10])
+    # empty strings and a lone blank at both ends, a 3006-byte string, an overlong `C1 A6` start of `foobar`, 3000
+    # short random strings, and C2 data: through the default route (K2c for `foo(bar|baz)`) and through K2 alone
+    more = [b"", b"", b" ", b"foobar", b"x" * 3000 + b"foobaz", b"", b"fooba", b"\xc1\xa6oobar fooba!"]
+    rng = np.random.default_rng(3)
+    more += [bytes(rng.integers(0x20, 0x7F, size=int(k), dtype=np.uint8)) for k in rng.integers(0, 300, size=3000)]
+    more += [b"foobaz", b"", b""]
+    sets = [pack(more), synth.gen_c2(40000)]
+    for sparse in ("1", "0"):
+        monkeypatch.setenv("FX_SPARSE", sparse)
+        for pat, op in [(b"foo(bar|baz)", "in"), (rb"\d{3}-\d{4}", "match"), (b"[a-z]+", "in"), (b"a*", "in"), (b"x*y+", "match")]:
+            p = fx.Pattern(pat, op)
+            for b_, o_ in sets:
+                got = p.in_batch(b_, o_) if op == "in" else p.match_batch(b_, o_)
+                info = p.info()
+                assert info["sparse_used"] == (info["sparse"] if sparse == "1" else 0)
+                exp = oracle_bool(pat, op, b_, offsets=o_)
+                assert np.array_equal(got, exp), (sparse, pat, op, np.nonzero(got != exp)[0][:10])
+    monkeypatch.delenv("FX_SPARSE")
     for pat in [b"[a-z]+", b"o+b", b"foobar", b"(foo|y+)$", b"^", b"\\s\\S+", b"aa[bc]", synth.PATTERNS["c3"]]:
         p = fx.Pattern(pat, "regex")
         f, t = p.regex_batch(buf, off)
@@ -394,26 +412,6 @@ def test_sparse_start_kernel(monkeypatch):
     monkeypatch.delenv("FX_SPARSE_MAX_FIRST")
     assert fx.Pattern(b"foo(bar|baz)", "in").info()["sparse"] == 1     # the C2 pattern takes this path by default
     assert fx.Pattern(rb"\w+@\w+", "in").info()["sparse"] == 0
-
-
-@pytest.mark.parametrize("form", ["1", "2"])
-def test_alternative_ragged_forms(monkeypatch, form):
-    """K2s (streaming windows, form 1) and K2p (length-balanced pairs, form 2) against the oracle"""
-    rng = np.random.default_rng(3)
-    strings = [b"", b"", b" ", b"foobar", b"x" * 3000 + b"foobaz", b"", b"fooba", b"\xc1\xa6oobar fooba!"]
-    strings += [bytes(rng.integers(0x20, 0x7F, size=int(k), dtype=np.uint8)) for k in rng.integers(0, 300, size=3000)]
-    strings += [b"foobaz", b"", b""]
-    buf, off = pack(strings)
-    buf2, off2 = synth.gen_c2(40000)
-    for window in ("64", "1024", "100000"):
-        monkeypatch.setenv("FX_RAGGED_FORM", form)
-        monkeypatch.setenv("FX_WINDOW", window)
-        for pat, op in [(b"foo(bar|baz)", "in"), (rb"\d{3}-\d{4}", "match"), (b"[a-z]+", "in"), (b"a*", "in"), (b"x*y+", "match")]:
-            p = fx.Pattern(pat, op)
-            for b_, o_ in ((buf, off), (buf2, off2)):
-                got = p.in_batch(b_, o_) if op == "in" else p.match_batch(b_, o_)
-                exp = oracle_bool(pat, op, b_, offsets=o_)
-                assert np.array_equal(got, exp), (window, pat, op, np.nonzero(got != exp)[0][:10])
 
 
 def test_buffer_windows_like_two_gpus():

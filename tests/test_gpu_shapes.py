@@ -319,22 +319,13 @@ def test_ragged_batch_past_4_gib(device, monkeypatch):
     h.close()
     del hbuf, hoff, got
 
-    # sub-batches at large offsets: a slice of the offsets with the whole buffer (offsets are absolute positions)
-    # for the forms too slow, or too rarely chosen, for the whole batch
+    # a sub-batch at large offsets: a slice of the offsets with the whole buffer (offsets are absolute positions)
+    # for the NFA engine, too slow for the whole batch
     lo = straddle[B32] - 1500
     sub = R.off[lo:lo + 3001]
     ns = 3000
     assert int(sub[0].item()) < B32 < int(sub[-1].item())
     so = torch.empty(ns, dtype=torch.uint8, device="cuda")
-    monkeypatch.setenv("FX_SPARSE", "0")
-    for form in ("1", "2"):
-        monkeypatch.setenv("FX_RAGGED_FORM", form)
-        for pat, op, exp in ((C2, "in", exp_in), (C1, "match", exp_match)):
-            so.fill_(7)
-            getattr(fx.Pattern(pat, op), op + "_batch_dev")(R.buf, sub, ns, total, so)
-            assert torch.equal(so, exp[lo:lo + ns]), (form, op)
-    monkeypatch.delenv("FX_RAGGED_FORM")
-    monkeypatch.delenv("FX_SPARSE")
     monkeypatch.setenv("FX_STATE_CAP", "3")                          # the NFA engine
     for pat, op, exp in ((C2, "in", exp_in), (C1, "match", exp_match)):
         e = fx.Pattern(pat, op)
