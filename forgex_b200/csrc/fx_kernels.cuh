@@ -981,24 +981,47 @@ __device__ __forceinline__ uint32_t first_mask(const SparseParams& sp, uint32_t 
     if (HIGH) m |= w;
     return m;
 }
+// TWO: the bytes of w that may follow the first byte turn into zero bytes: the second byte, and, when lead bytes can
+// follow (second_high), every byte >= 0x80.  The PRMT selector of lead_sel() replicates each byte's bit 7 over the
+// byte (0xBA98), or gives zero (0x4444 picks the zero operand's byte 0).
+__device__ __forceinline__ uint32_t lead_sel(const SparseParams& sp) { return sp.second_high ? 0xBA98u : 0x4444u; }
+template <bool LEAD>
+__device__ __forceinline__ uint32_t second_zero(const SparseParams& sp, uint32_t w, uint32_t sel) {
+    uint32_t z = w ^ sp.second;
+    if (LEAD) {
+        uint32_t s;
+        asm("prmt.b32 %0, %1, 0, %2;" : "=r"(s) : "r"(w), "r"(sel));
+        z &= ~s;
+    }
+    return z;
+}
+// TWO: bit 7 of byte j set when byte j of w is the first byte and the byte after it may follow: z = second_zero of
+// w, z_next = second_zero of the word after w (only its byte 0 is used).  Byte j of t is zero exactly for such a
+// pair; the zero-byte test also flags a 0x01 byte of t above a zero byte (a borrow neighbour), so a word with a pair
+// is always flagged and a word without one never is.
+__device__ __forceinline__ uint32_t pair_mask(const SparseParams& sp, uint32_t w, uint32_t z, uint32_t z_next) {
+    const uint32_t t = (w ^ sp.add_lo[0]) | __funnelshift_r(z, z_next, 8);
+    return (t - 0x01010101u) & ~t;
+}
 // Sweep filter for one 32-byte unit: non-zero when the unit may hold a candidate.  TWO (with NR = -1): a candidate
-// is the first byte FOLLOWED BY the second byte (or by a lead byte, if lead bytes can follow); whatever follows the
-// unit's last byte is assumed to match.  `seen` collects the OR of the unit's words (bytes >= 0x80 in the tile?).
+// is the first byte FOLLOWED BY the second byte (or by a lead byte, if lead bytes can follow); z_next is second_zero
+// of the word after the unit (0 where that word is not known: the byte after the unit is assumed to match).  `seen`
+// collects the OR of the unit's words (bytes >= 0x80 in the tile?).
 template <int NR, bool HIGH, bool TWO>
-__device__ __forceinline__ uint32_t unit_any(const SparseParams& sp, const uint4& a, const uint4& b, uint32_t& seen) {
+__device__ __forceinline__ uint32_t unit_any(const SparseParams& sp, const uint4& a, const uint4& b, uint32_t& seen,
+                                             uint32_t z_next = 0u) {
     const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
     const uint32_t all = w[0] | w[1] | w[2] | w[3] | w[4] | w[5] | w[6] | w[7];
     seen |= all;
     uint32_t any = 0;
     if (TWO) {
-        uint32_t z2_next = 0xFFFFFFFFu;
+        const uint32_t sel = lead_sel(sp);
 #pragma unroll
         for (int k = 7; k >= 0; k--) {
-            const uint32_t x1 = w[k] ^ sp.add_lo[0], x2 = w[k] ^ sp.second;
-            uint32_t z2 = (x2 - 0x01010101u) & ~x2;
-            if (!HIGH) z2 |= w[k] & sp.second_high;            // (with HIGH every byte >= 0x80 makes the unit pass anyway)
-            any |= (x1 - 0x01010101u) & ~x1 & __funnelshift_r(z2, z2_next, 8);   // first byte at j and second byte at j + 1
-            z2_next = z2;
+            // with HIGH every byte >= 0x80 makes the unit pass anyway: lead bytes inside the unit need no test
+            const uint32_t z = second_zero<!HIGH>(sp, w[k], sel);
+            any |= pair_mask(sp, w[k], z, z_next);
+            z_next = z;
         }
         if (HIGH) any |= all;
     } else {
@@ -1125,7 +1148,8 @@ __device__ __noinline__ void sparse_run_starts(const KParams& p, const SparsePar
 // Phase U: `count` (<= 32) queued units {tile, high << 31, unit number (64 bit) from the tile's 32-byte aligned base},
 // one per lane.  Candidates are taken in rounds (round k = every lane's k-th candidate); a candidate survives unless
 // two bytes prove the start dead.  Survivors go to the start queue (sqn = its fill level), which is run when full.
-template <int KIND, int NR, bool HIGH>
+// TWO: the candidates are the byte pairs of the sweep filter (the two table steps still confirm each one).
+template <int KIND, int NR, bool HIGH, bool TWO>
 __device__ __noinline__ int sparse_run_units(const KParams& p, const SparseParams& sp, uint32_t s_table, uint32_t s_cmap,
                                              const SparseCtx& c, int count, int sqn) {
     const Table<KIND> T = sparse_table<KIND>(sp, s_table, s_cmap);
@@ -1144,11 +1168,25 @@ __device__ __noinline__ int sparse_run_units(const KParams& p, const SparseParam
         const uintptr_t gbuf = reinterpret_cast<uintptr_t>(c.buf);
         const uintptr_t ua = ((gbuf + (uintptr_t)t0) & ~(uintptr_t)31) + ((((uintptr_t)e.w << 32) | e.z) << 5);
         const uint4 v0 = __ldg(reinterpret_cast<const uint4*>(ua)), v1 = __ldg(reinterpret_cast<const uint4*>(ua + 16));
-        cand = pack_byte_flags(first_mask<NR, HIGH>(sp, v0.x)) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v0.y)) << 4) |
-               (pack_byte_flags(first_mask<NR, HIGH>(sp, v0.z)) << 8) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v0.w)) << 12) |
-               (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.x)) << 16) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.y)) << 20) |
-               (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.z)) << 24) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.w)) << 28);
         P = (int64_t)ua - (int64_t)gbuf;
+        if (TWO) {
+            // the byte after the unit, if it is in the tile; else a start on the unit's last byte is the last byte of
+            // the tile's last string, and the byte is assumed to match
+            const uint32_t sel = lead_sel(sp);
+            uint32_t z_next = P + 32 < tend ? second_zero<true>(sp, __ldg(reinterpret_cast<const uint8_t*>(ua + 32)), sel) : 0u;
+            const uint32_t w[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
+#pragma unroll
+            for (int k = 7; k >= 0; k--) {
+                const uint32_t z = second_zero<true>(sp, w[k], sel);
+                cand |= pack_byte_flags(pair_mask(sp, w[k], z, z_next) | (HIGH ? w[k] : 0u)) << (4 * k);
+                z_next = z;
+            }
+        } else {
+            cand = pack_byte_flags(first_mask<NR, HIGH>(sp, v0.x)) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v0.y)) << 4) |
+                   (pack_byte_flags(first_mask<NR, HIGH>(sp, v0.z)) << 8) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v0.w)) << 12) |
+                   (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.x)) << 16) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.y)) << 20) |
+                   (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.z)) << 24) | (pack_byte_flags(first_mask<NR, HIGH>(sp, v1.w)) << 28);
+        }
         if (P < t0) cand &= 0xFFFFFFFFu << (int)(t0 - P);
         if (P + 32 > tend) cand &= (P >= tend) ? 0u : (0xFFFFFFFFu >> (int)(P + 32 - tend));
     }
@@ -1185,6 +1223,50 @@ __device__ __noinline__ int sparse_run_units(const KParams& p, const SparseParam
 
 // 4 CTAs per SM, 4 rows (4 KB per warp) in flight: the best of the measured combinations (DESIGN.md section 5)
 static constexpr int SPARSE_CTAS_PER_SM = 4, SPARSE_ROWS = 4;
+
+// One group of the sweep: rows r .. r + SPARSE_ROWS - 1 (32 units each) of a segment of `lim` units that starts at
+// `sbase`.  Returns bit k set when this lane's unit in row r + k passed the filter.  WHOLE: every unit of the group lies
+// in the segment, so nothing is bounds-tested or zeroed (all groups but a tile's last).
+template <int NR, bool HIGH, bool TWO, bool WHOLE>
+__device__ __forceinline__ uint32_t sweep_group(const SparseParams& sp, uintptr_t sbase, int r, int lim, uint32_t& seen) {
+    const int lane = threadIdx.x & 31;
+    uint4 va[SPARSE_ROWS], vb[SPARSE_ROWS];
+#pragma unroll
+    for (int k = 0; k < SPARSE_ROWS; k++) {            // all loads first: SPARSE_ROWS KB per warp in flight
+        const int u = ((r + k) << 5) + lane;
+        const uintptr_t a = sbase + ((uintptr_t)(uint32_t)u << 5);
+        if (WHOLE || u < lim) {
+            va[k] = ldg_nc_v4(reinterpret_cast<const void*>(a));
+            vb[k] = ldg_nc_v4(reinterpret_cast<const void*>(a + 16));
+        } else {
+            va[k] = make_uint4(0, 0, 0, 0); vb[k] = va[k];
+        }
+    }
+    // TWO: the first word of the next unit is in lane + 1 of the same row, or for lane 31 in lane 0 of the next row.
+    // After the group's last row and after the segment's last unit the next unit is not loaded: it is assumed to match.
+    uint32_t zn[SPARSE_ROWS];
+    if (TWO) {
+        const uint32_t sel = lead_sel(sp);
+        uint32_t z0[SPARSE_ROWS];
+#pragma unroll
+        for (int k = 0; k < SPARSE_ROWS; k++) z0[k] = second_zero<true>(sp, va[k].x, sel);
+#pragma unroll
+        for (int k = 0; k < SPARSE_ROWS; k++) {
+            const uint32_t give = lane != 0 ? z0[k] : k + 1 < SPARSE_ROWS ? z0[k + 1] : 0u;
+            zn[k] = __shfl_sync(0xffffffffu, give, (lane + 1) & 31);
+            if (!WHOLE && ((r + k) << 5) + lane + 1 >= lim) zn[k] = 0u;
+        }
+    }
+    uint32_t bits = 0;
+#pragma unroll
+    for (int k = 0; k < SPARSE_ROWS; k++) {
+        const int u = ((r + k) << 5) + lane;
+        const uint32_t h = (WHOLE || u < lim) ? unit_any<NR, HIGH, TWO>(sp, va[k], vb[k], seen, TWO ? zn[k] : 0u) : 0u;
+        bits |= (h ? 1u : 0u) << k;
+    }
+    return bits;
+}
+
 template <int KIND, int NR, bool HIGH, bool TWO>
 __global__ void __launch_bounds__(256, SPARSE_CTAS_PER_SM) k_in_sparse(KParams p, SparseParams sp, const uint8_t* __restrict__ buf,
                                                                      const int64_t* __restrict__ offsets, int64_t n, int64_t total,
@@ -1255,27 +1337,15 @@ __global__ void __launch_bounds__(256, SPARSE_CTAS_PER_SM) k_in_sparse(KParams p
             if (st == ST_SWEEP) {
                 // ---- S: up to 32 rows of 32 units, SPARSE_ROWS rows (SPARSE_ROWS KB per warp) in flight ----
                 const int64_t left = nunits - seg;
-                nrows = (int)((left < 1024 ? left : 1024) + 31) >> 5;
+                const int lim = (int)(left < 1024 ? left : 1024);  // units in this segment
+                const uintptr_t sbase = ubase + ((uintptr_t)seg << 5);
+                nrows = (lim + 31) >> 5;
                 hitbits = 0;
                 uint32_t seen = 0;
-                for (int r = 0; r < nrows; r += SPARSE_ROWS) {
-                    uint4 va[SPARSE_ROWS], vb[SPARSE_ROWS];
-#pragma unroll
-                    for (int k = 0; k < SPARSE_ROWS; k++) {        // all loads first: SPARSE_ROWS KB per warp in flight
-                        const int64_t u = seg + ((int64_t)(r + k) << 5) + lane;
-                        va[k] = make_uint4(0, 0, 0, 0); vb[k] = va[k];
-                        if (u < nunits && r + k < nrows) {
-                            va[k] = ldg_nc_v4(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5)));
-                            vb[k] = ldg_nc_v4(reinterpret_cast<const void*>(ubase + ((uintptr_t)u << 5) + 16));
-                        }
-                    }
-#pragma unroll
-                    for (int k = 0; k < SPARSE_ROWS; k++) {
-                        const int64_t u = seg + ((int64_t)(r + k) << 5) + lane;
-                        const uint32_t h = (u < nunits && r + k < nrows) ? unit_any<NR, HIGH, TWO>(sp, va[k], vb[k], seen) : 0u;
-                        hitbits |= (h ? 1u : 0u) << (r + k);
-                    }
-                }
+                int r = 0;
+                for (; ((r + SPARSE_ROWS) << 5) <= lim; r += SPARSE_ROWS)
+                    hitbits |= sweep_group<NR, HIGH, TWO, true>(sp, sbase, r, lim, seen) << r;
+                if (r < nrows) hitbits |= sweep_group<NR, HIGH, TWO, false>(sp, sbase, r, lim, seen) << r;
                 high = high || __any_sync(FULL, (seen & 0x80808080u) != 0);   // (bytes next to the tile are counted in: harmless)
                 st = seg == 0 ? ST_STRINGS : ST_PUSH;              // the strings' own results are written before any unit is queued
                 it = 0;
@@ -1331,7 +1401,7 @@ __global__ void __launch_bounds__(256, SPARSE_CTAS_PER_SM) k_in_sparse(KParams p
         // ---- outer loop: run a queue (the only calls of the kernel) ----
         if (uqn >= 32 || (drain && uqn > 0)) {
             const int run = uqn < 32 ? uqn : 32;
-            sqn = sparse_run_units<KIND, NR, HIGH>(*sh_p, *sh_sp, T.s_table, T.s_cmap, *sh_c, run, sqn);
+            sqn = sparse_run_units<KIND, NR, HIGH, TWO>(*sh_p, *sh_sp, T.s_table, T.s_cmap, *sh_c, run, sqn);
             if (lane < uqn - run) { const uint4 x = s_units[run + lane]; s_units[lane] = x; }
             uqn -= run;
             __syncwarp();
