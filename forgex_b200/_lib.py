@@ -25,6 +25,7 @@ SYMBOLS = [
     "fx_statemap_window_dev", "fx_statemap_combine", "fx_statemap_back_dev",
     "fx_match_fixed", "fx_in_fixed", "fx_match_batch", "fx_in_batch", "fx_regex_batch", "fx_regex_buffer",
     "fx_regex_count_batch_dev", "fx_regex_buffer_all_dev", "fx_regex_count_batch", "fx_regex_buffer_all",
+    "fx_regex_all_batch_work_bytes", "fx_regex_all_batch_dev", "fx_regex_all_batch",
     "fx_in", "fx_match", "fx_regex", "fx_in_value", "fx_match_value", "fx_regex_sub", "fx_launch_count",
 ]
 
@@ -97,6 +98,10 @@ def lib():
     L.fx_regex_buffer_all_dev.argtypes = [vp, u8p, i64, vp, vp, i64, C.POINTER(i64), vp, vp]
     L.fx_regex_count_batch.argtypes = [vp, u8p, vp, i64, vp]
     L.fx_regex_buffer_all.argtypes = [vp, u8p, i64, vp, vp, i64, C.POINTER(i64)]
+    L.fx_regex_all_batch_work_bytes.restype = i64
+    L.fx_regex_all_batch_work_bytes.argtypes = [i64]
+    L.fx_regex_all_batch_dev.argtypes = [vp, u8p, vp, i64, i64, vp, vp, vp, i64, vp, vp]
+    L.fx_regex_all_batch.argtypes = [vp, u8p, vp, i64, vp, vp, vp, i64]
     L.fx_in.argtypes = [C.c_char_p, i64, C.c_char_p, i64, C.POINTER(C.c_int)]
     L.fx_match.argtypes = [C.c_char_p, i64, C.c_char_p, i64, C.POINTER(C.c_int)]
     L.fx_regex.argtypes = [C.c_char_p, i64, C.c_char_p, i64, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64),

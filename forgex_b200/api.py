@@ -10,6 +10,8 @@
     is_valid_regex(pattern)                is_valid_regex(pattern)
     (new) one pattern against N strings    Pattern(...).match_fixed / in_fixed / match_batch / in_batch / regex_batch
     (new) one pattern, one huge buffer     Pattern(...).regex_buffer
+    (new) every match, the way a caller    Pattern(...).regex_count_batch (matches per string),
+          loops regex on text(to+1:)       regex_all_batch (every span of every string), regex_buffer_all (one buffer)
 
 Same argument meaning and error behaviour as the reference: an invalid pattern makes the operators
 return False, and makes regex return res=b'', length=0, from=to=-9999 with the SYNTAX_* status and
@@ -263,6 +265,20 @@ class Pattern:
         k = min(cnt.value, capacity)
         return f[:k], t[:k], cnt.value
 
+    def regex_all_batch(self, buf, offsets, capacity=1 << 20):
+        """every match of every string: (rows[n + 1], from[], to[]).  String i's spans are from/to[rows[i]:rows[i + 1]],
+        1-based inclusive in the string's own coordinates; rows is complete, the spans are cut to min(rows[-1], capacity)"""
+        buf = np.ascontiguousarray(buf, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        n = len(offsets) - 1
+        rows = np.zeros(n + 1, dtype=np.int64)
+        f = np.zeros(max(capacity, 1), dtype=np.int64)
+        t = np.zeros(max(capacity, 1), dtype=np.int64)
+        _check(L.lib().fx_regex_all_batch(self.h, _ptr(buf), _ptr(offsets), n, _ptr(rows), _ptr(f), _ptr(t), capacity),
+               "fx_regex_all_batch")
+        k = min(int(rows[-1]), capacity)
+        return rows, f[:k], t[:k]
+
     # ---- device-resident calls (torch CUDA tensors; nothing is copied; runs on torch's current stream) ----
     @staticmethod
     def _stream():
@@ -310,6 +326,19 @@ class Pattern:
         _check(L.lib().fx_regex_buffer_all_dev(self.h, _ptr(d_buf), length, _ptr(d_from), _ptr(d_to), capacity, C.byref(cnt),
                                                _ptr(d_work), self._stream()), "fx_regex_buffer_all_dev")
         return cnt.value
+
+    @staticmethod
+    def all_batch_work_bytes(n):
+        """size of the device scratch fx_regex_all_batch_dev needs for a batch of `n` strings"""
+        return int(L.lib().fx_regex_all_batch_work_bytes(n))
+
+    def regex_all_batch_dev(self, d_buf, d_offsets, n, total, d_rows, d_from, d_to, capacity, d_work):
+        """rows into d_rows (n + 1 int64), the spans below `capacity` into d_from / d_to; asynchronous"""
+        assert d_work.numel() * d_work.element_size() >= self.all_batch_work_bytes(n), "d_work is too small"
+        _check(L.lib().fx_regex_all_batch_dev(self.h, _ptr(d_buf), _ptr(d_offsets), n, total, _ptr(d_rows),
+                                              _ptr(d_from) if d_from is not None else None,
+                                              _ptr(d_to) if d_to is not None else None, capacity, _ptr(d_work),
+                                              self._stream()), "fx_regex_all_batch_dev")
 
     def buffer_scan_dev(self, d_window, window_len, start_lo, start_hi, origin, is_first, is_last, d_best):
         _check(L.lib().fx_buffer_scan_dev(self.h, _ptr(d_window), window_len, start_lo, start_hi, origin,

@@ -1067,6 +1067,46 @@ int grow(T*& ptr, size_t& cap, size_t need_bytes) {
     return FX_OK;
 }
 
+// k_regex_count over a ragged batch of n > 0 strings: the counts into `counts`, or with WRITE the spans below
+// `capacity` into d_from / d_to at the row offsets `counts` holds
+template <bool WRITE>
+int launch_regex_count(fx_pattern* p, const uint8_t* d_buf, const int64_t* d_offsets, int64_t n, int64_t* counts,
+                       int64_t* d_from, int64_t* d_to, int64_t capacity, cudaStream_t s) {
+    int rc;
+    Plan pl;
+    if ((rc = make_plan(p, pl))) return rc;
+    SpanParams sp;
+    memset(&sp, 0, sizeof(sp));
+    long long want = (n + 255) / 256, cap = (long long)p->dev.sm_count * 16;
+    const int grid = (int)(want < cap ? want : cap);
+    if (p->prog.has_span && env_int("FX_SPAN_LINEAR", 1)) {
+        fill_span_params(p, sp);
+        k_regex_count<true, WRITE><<<grid, 256, 0, s>>>(pl.kp, sp, d_buf, d_offsets, n, counts, d_from, d_to, capacity);
+    } else {
+        k_regex_count<false, WRITE><<<grid, 256, 0, s>>>(pl.kp, sp, d_buf, d_offsets, n, counts, d_from, d_to, capacity);
+    }
+    g_launches++;
+    return cuda_status(cudaGetLastError());
+}
+
+// blocks of the row-offset scan for n values: one per FX_SCAN_TILE values, at most FX_SCAN_MAX_BLOCKS
+int64_t scan_blocks(int64_t n) {
+    const int64_t b = (n + FX_SCAN_TILE - 1) / FX_SCAN_TILE;
+    return b < 1 ? 1 : (b > FX_SCAN_MAX_BLOCKS ? FX_SCAN_MAX_BLOCKS : b);
+}
+
+// inclusive scan of x[0, n) in place (n > 0); `sums`: scan_blocks(n) words of scratch
+int launch_scan_i64(int64_t* x, int64_t n, int64_t* sums, cudaStream_t s) {
+    const int64_t blocks = scan_blocks(n);
+    const int64_t tiles = ((n + blocks - 1) / blocks + FX_SCAN_TILE - 1) / FX_SCAN_TILE;
+    const int64_t chunk = tiles * FX_SCAN_TILE;
+    k_scan_i64_sums<<<(int)blocks, FX_SCAN_THREADS, 0, s>>>(x, n, chunk, sums);
+    k_scan_i64_carry<<<1, FX_SCAN_MAX_BLOCKS, 0, s>>>(sums, (int)blocks);
+    k_scan_i64_apply<<<(int)blocks, FX_SCAN_THREADS, 0, s>>>(x, n, chunk, sums);
+    g_launches += 3;
+    return cuda_status(cudaGetLastError());
+}
+
 }  // namespace
 
 // =============================================================================================
@@ -1540,20 +1580,27 @@ int fx_regex_count_batch_dev(fx_pattern* p, const uint8_t* d_buf, const int64_t*
     if (n < 0 || total_bytes < 0 || !d_counts) return FX_ERR_BAD_ARGUMENT;
     if (n == 0) return FX_OK;
     if (p->prog.nfa_engine) return FX_ERR_DFA_STATE_CAP;        // (counting needs the table engine)
-    Plan pl;
-    if ((rc = make_plan(p, pl))) return rc;
-    SpanParams sp;
-    memset(&sp, 0, sizeof(sp));
-    long long want = (n + 255) / 256, cap = (long long)p->dev.sm_count * 16;
-    const int grid = (int)(want < cap ? want : cap);
-    if (p->prog.has_span && env_int("FX_SPAN_LINEAR", 1)) {
-        fill_span_params(p, sp);
-        k_regex_count<true><<<grid, 256, 0, (cudaStream_t)stream>>>(pl.kp, sp, d_buf, d_offsets, n, d_counts);
-    } else {
-        k_regex_count<false><<<grid, 256, 0, (cudaStream_t)stream>>>(pl.kp, sp, d_buf, d_offsets, n, d_counts);
-    }
-    g_launches++;
-    return cuda_status(cudaGetLastError());
+    return launch_regex_count<false>(p, d_buf, d_offsets, n, d_counts, nullptr, nullptr, 0, (cudaStream_t)stream);
+}
+
+int64_t fx_regex_all_batch_work_bytes(int64_t n) { return 8 * scan_blocks(n < 0 ? 0 : n); }
+
+// Every match of every string: counts into d_rows + 1, d_rows[0] = 0, the inclusive scan of d_rows[1..n] in place, then
+// (capacity > 0) the span pass.  Asynchronous on `stream`: no host sync, nothing read back.
+int fx_regex_all_batch_dev(fx_pattern* p, const uint8_t* d_buf, const int64_t* d_offsets, int64_t n, int64_t total_bytes,
+                           int64_t* d_rows, int64_t* d_from, int64_t* d_to, int64_t capacity, void* d_work, void* stream) {
+    int rc = check_ready(p, FX_OP_REGEX);
+    if (rc) return rc;
+    if (n < 0 || total_bytes < 0 || capacity < 0 || !d_rows || !d_work || (capacity > 0 && (!d_from || !d_to)))
+        return FX_ERR_BAD_ARGUMENT;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (n == 0) return cuda_status(cudaMemsetAsync(d_rows, 0, 8, s));
+    if (p->prog.nfa_engine) return FX_ERR_DFA_STATE_CAP;
+    if ((rc = launch_regex_count<false>(p, d_buf, d_offsets, n, d_rows + 1, nullptr, nullptr, 0, s))) return rc;
+    CUDA_TRY(cudaMemsetAsync(d_rows, 0, 8, s));
+    if ((rc = launch_scan_i64(d_rows + 1, n, static_cast<int64_t*>(d_work), s))) return rc;
+    if (capacity == 0) return FX_OK;
+    return launch_regex_count<true>(p, d_buf, d_offsets, n, d_rows, d_from, d_to, capacity, s);
 }
 
 // One buffer: every match, in order.  d_from / d_to receive the first `capacity` spans (64-bit, 1-based inclusive, in
@@ -1705,6 +1752,33 @@ int fx_regex_count_batch(fx_pattern* p, const uint8_t* buf, const int64_t* offse
     if ((rc = grow(d.w_span, d.w_span_cap, (size_t)n * 8))) return rc;
     if ((rc = fx_regex_count_batch_dev(p, d.w_buf, d.w_off, n, total, d.w_span, nullptr))) return rc;
     CUDA_TRY(cudaMemcpyAsync(counts, d.w_span, (size_t)n * 8, cudaMemcpyDeviceToHost, 0));
+    CUDA_TRY(cudaStreamSynchronize(0));
+    return FX_OK;
+}
+// rows first (the _dev form with capacity 0), then the span pass for the min(rows[n], capacity) spans that come back:
+// the device holds no more span room than the answer needs
+int fx_regex_all_batch(fx_pattern* p, const uint8_t* buf, const int64_t* offsets, int64_t n, int64_t* rows, int64_t* from,
+                       int64_t* to, int64_t capacity) {
+    int rc = check_ready(p, FX_OP_REGEX);
+    if (rc) return rc;
+    if (n < 0 || capacity < 0 || !offsets || !rows || (capacity > 0 && (!from || !to))) return FX_ERR_BAD_ARGUMENT;
+    if (n == 0) { rows[0] = 0; return FX_OK; }
+    std::lock_guard<std::mutex> lock(p->mu);
+    DeviceTables& d = p->dev;
+    int64_t total = 0;
+    if ((rc = host_stage_ragged(p, buf, offsets, n, total))) return rc;
+    if ((rc = grow(d.w_span, d.w_span_cap, (size_t)(n + 1) * 8))) return rc;
+    if ((rc = grow(d.w_work, d.w_work_cap, (size_t)fx_regex_all_batch_work_bytes(n)))) return rc;
+    if ((rc = fx_regex_all_batch_dev(p, d.w_buf, d.w_off, n, total, d.w_span, nullptr, nullptr, 0, d.w_work, nullptr))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(rows, d.w_span, (size_t)(n + 1) * 8, cudaMemcpyDeviceToHost, 0));
+    CUDA_TRY(cudaStreamSynchronize(0));
+    const int64_t k = rows[n] < capacity ? rows[n] : capacity;
+    if (k == 0) return FX_OK;
+    if ((rc = grow(d.w_out, d.w_out_cap, (size_t)k * 16))) return rc;        // (w_out: the spans, as int64)
+    int64_t* d_from = reinterpret_cast<int64_t*>(d.w_out);
+    if ((rc = launch_regex_count<true>(p, d.w_buf, d.w_off, n, d.w_span, d_from, d_from + k, k, 0))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(from, d_from, (size_t)k * 8, cudaMemcpyDeviceToHost, 0));
+    CUDA_TRY(cudaMemcpyAsync(to, d_from + k, (size_t)k * 8, cudaMemcpyDeviceToHost, 0));
     CUDA_TRY(cudaStreamSynchronize(0));
     return FX_OK;
 }

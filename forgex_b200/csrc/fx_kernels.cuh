@@ -2911,21 +2911,107 @@ __device__ __forceinline__ void regex_once(const KParams& p, const SpanParams& s
     }
 }
 
-// number of matches per string of a ragged batch (one thread per string)
-template <bool SPAN>
+// number of matches per string of a ragged batch (one thread per string).  WRITE: the span pass of the batch form --
+// `counts` holds the row offsets instead (rows[n + 1], the counts' prefix sum behind rows[0] = 0, read only) and string
+// i's k-th match goes to out_from / out_to[rows[i] + k], 1-based in the string's own coordinates, for indices below
+// `capacity`; the loop stops there or after the string's rows[i + 1] - rows[i] matches.
+template <bool SPAN, bool WRITE = false>
 __global__ void __launch_bounds__(256) k_regex_count(KParams p, SpanParams sp, const uint8_t* __restrict__ buf,
-                                                     const int64_t* __restrict__ offsets, int64_t n, int64_t* __restrict__ counts) {
+                                                     const int64_t* __restrict__ offsets, int64_t n, int64_t* __restrict__ counts,
+                                                     int64_t* __restrict__ out_from = nullptr, int64_t* __restrict__ out_to = nullptr,
+                                                     int64_t capacity = 0) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const int64_t o0 = __ldg(offsets + i), o1 = __ldg(offsets + i + 1);
-        int64_t pos = 0, cnt = 0;
+        int64_t pos = 0, cnt = 0, end = 0;
+        if (WRITE) {
+            cnt = counts[i];
+            end = counts[i + 1] < capacity ? counts[i + 1] : capacity;
+        }
         for (;;) {
+            if (WRITE && cnt >= end) break;
             int64_t f, t;
             regex_once<SPAN>(p, sp, buf + o0 + pos, o1 - o0 - pos, f, t);
             if (f <= 0 || t <= 0) break;
+            if (WRITE) { out_from[cnt] = pos + f; out_to[cnt] = pos + t; }
             cnt++;
             pos += t;
         }
-        counts[i] = cnt;
+        if (!WRITE) counts[i] = cnt;
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Inclusive scan of int64 in place (the row offsets of the all-matches batch form), on a fixed grid of at most
+// FX_SCAN_MAX_BLOCKS blocks: block b owns x[b * chunk, (b + 1) * chunk), chunk a multiple of FX_SCAN_TILE.
+// k_scan_i64_sums writes each block's sum to sums[b], k_scan_i64_carry (one block) turns sums[] into exclusive prefixes,
+// k_scan_i64_apply rescans each range tile by tile from its prefix.  Scratch: sums[], 8 bytes per block.
+// ---------------------------------------------------------------------------------------------
+constexpr int FX_SCAN_THREADS = 256, FX_SCAN_ITEMS = 4, FX_SCAN_TILE = FX_SCAN_THREADS * FX_SCAN_ITEMS, FX_SCAN_MAX_BLOCKS = 1024;
+
+// inclusive scan of one value per thread over a block of THREADS threads; *total = the block's sum.
+// warp_sums: THREADS / 32 words of shared memory, free again when this returns.
+template <int THREADS>
+__device__ __forceinline__ long long block_scan_i64(long long v, long long* warp_sums, long long& total) {
+    static_assert(THREADS % 32 == 0 && THREADS <= 1024, "one warp scans the warp sums");
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    for (int d = 1; d < 32; d <<= 1) {
+        const long long u = __shfl_up_sync(0xFFFFFFFFu, v, d);
+        if (lane >= d) v += u;
+    }
+    if (lane == 31) warp_sums[w] = v;
+    __syncthreads();
+    if (w == 0) {
+        long long s = lane < THREADS / 32 ? warp_sums[lane] : 0;
+        for (int d = 1; d < 32; d <<= 1) {
+            const long long u = __shfl_up_sync(0xFFFFFFFFu, s, d);
+            if (lane >= d) s += u;
+        }
+        if (lane < THREADS / 32) warp_sums[lane] = s;
+    }
+    __syncthreads();
+    if (w > 0) v += warp_sums[w - 1];
+    total = warp_sums[THREADS / 32 - 1];
+    __syncthreads();
+    return v;
+}
+
+__global__ void __launch_bounds__(FX_SCAN_THREADS) k_scan_i64_sums(const int64_t* __restrict__ x, int64_t n, int64_t chunk,
+                                                                   int64_t* __restrict__ sums) {
+    __shared__ long long ws[FX_SCAN_THREADS / 32];
+    const int64_t lo = (int64_t)blockIdx.x * chunk, hi = lo + chunk < n ? lo + chunk : n;
+    long long s = 0;
+    for (int64_t k = lo + threadIdx.x; k < hi; k += FX_SCAN_THREADS) s += x[k];
+    long long total;
+    block_scan_i64<FX_SCAN_THREADS>(s, ws, total);
+    if (threadIdx.x == 0) sums[blockIdx.x] = total;
+}
+
+__global__ void __launch_bounds__(FX_SCAN_MAX_BLOCKS) k_scan_i64_carry(int64_t* __restrict__ sums, int nblocks) {
+    __shared__ long long ws[FX_SCAN_MAX_BLOCKS / 32];
+    const long long v = (int)threadIdx.x < nblocks ? sums[threadIdx.x] : 0;
+    long long total;
+    const long long incl = block_scan_i64<FX_SCAN_MAX_BLOCKS>(v, ws, total);
+    if ((int)threadIdx.x < nblocks) sums[threadIdx.x] = incl - v;
+}
+
+__global__ void __launch_bounds__(FX_SCAN_THREADS) k_scan_i64_apply(int64_t* __restrict__ x, int64_t n, int64_t chunk,
+                                                                    const int64_t* __restrict__ sums) {
+    __shared__ long long ws[FX_SCAN_THREADS / 32];
+    const int64_t lo = (int64_t)blockIdx.x * chunk, hi = lo + chunk < n ? lo + chunk : n;
+    long long carry = sums[blockIdx.x];
+    for (int64_t t0 = lo; t0 < hi; t0 += FX_SCAN_TILE) {
+        const int64_t base = t0 + (int64_t)threadIdx.x * FX_SCAN_ITEMS;
+        long long v[FX_SCAN_ITEMS];
+#pragma unroll
+        for (int j = 0; j < FX_SCAN_ITEMS; j++) v[j] = base + j < hi ? x[base + j] : 0;
+#pragma unroll
+        for (int j = 1; j < FX_SCAN_ITEMS; j++) v[j] += v[j - 1];
+        long long total;
+        const long long before = block_scan_i64<FX_SCAN_THREADS>(v[FX_SCAN_ITEMS - 1], ws, total) - v[FX_SCAN_ITEMS - 1] + carry;
+#pragma unroll
+        for (int j = 0; j < FX_SCAN_ITEMS; j++)
+            if (base + j < hi) x[base + j] = v[j] + before;
+        carry += total;
     }
 }
 

@@ -13,7 +13,7 @@
 !                             a flat buffer + offsets (variable length; trailing blanks are text to Forgex)
 !     regex_batch             (from, to) per string
 !     regex_buffer            one pattern against one huge buffer, 64-bit positions
-!     regex_count_batch / regex_buffer_all   every match, the way a caller loops regex on text(to+1:)
+!     regex_count_batch / regex_all_batch / regex_buffer_all   every match, the way a caller loops regex on text(to+1:)
 !     is_valid_regex_batch    is_valid_regex over an array of patterns, one call
 !     *_dev / window forms    device pointers (type(c_ptr)) + a CUDA stream, for CUDA Fortran / OpenACC hosts and for
 !                             a text that is split across GPUs
@@ -45,7 +45,8 @@ module forgex_b200_m
       procedure :: free    => pattern__free
    end type fx_pattern_t
 
-   public :: match_batch, in_batch, regex_batch, regex_buffer, regex_count_batch, regex_buffer_all, is_valid_regex_batch
+   public :: match_batch, in_batch, regex_batch, regex_buffer, regex_count_batch, regex_all_batch, regex_buffer_all, &
+             is_valid_regex_batch
 
    interface match_batch
       module procedure :: match_batch__fixed, match_batch__ragged
@@ -197,6 +198,16 @@ module forgex_b200_m
          integer(c_int64_t), intent(out) :: from(*), to(*), count
          integer(c_int) :: status
       end function
+      function fx_regex_all_batch(p, buf, offsets, n, rows, from, to, capacity) bind(c, name='fx_regex_all_batch') result(status)
+         import :: c_ptr, c_char, c_int64_t, c_int
+         type(c_ptr), value :: p
+         character(kind=c_char), intent(in) :: buf(*)
+         integer(c_int64_t), intent(in) :: offsets(*)
+         integer(c_int64_t), value :: n, capacity
+         integer(c_int64_t), intent(out) :: rows(*)
+         integer(c_int64_t), intent(inout) :: from(*), to(*)      ! only the first min(rows(n+1), capacity) are written
+         integer(c_int) :: status
+      end function
       ! ---- device-pointer forms: buffers are type(c_ptr) device addresses (c_loc of a CUDA Fortran device array,
       !      acc_deviceptr, ...), stream = a cudaStream_t as c_ptr (c_null_ptr = default stream); asynchronous ----
       function fx_match_fixed_dev(p, d_buf, n, stride, d_out, stream) bind(c, name='fx_match_fixed_dev') result(status)
@@ -252,6 +263,18 @@ module forgex_b200_m
          type(c_ptr), value :: p, d_buf, d_from, d_to, d_work, stream
          integer(c_int64_t), value :: length, capacity
          integer(c_int64_t), intent(out) :: count          ! host memory
+         integer(c_int) :: status
+      end function
+      function fx_regex_all_batch_work_bytes(n) bind(c, name='fx_regex_all_batch_work_bytes') result(nbytes)
+         import :: c_int64_t
+         integer(c_int64_t), value :: n
+         integer(c_int64_t) :: nbytes
+      end function
+      function fx_regex_all_batch_dev(p, d_buf, d_offsets, n, total_bytes, d_rows, d_from, d_to, capacity, d_work, stream) &
+            bind(c, name='fx_regex_all_batch_dev') result(status)
+         import :: c_ptr, c_int64_t, c_int
+         type(c_ptr), value :: p, d_buf, d_offsets, d_rows, d_from, d_to, d_work, stream
+         integer(c_int64_t), value :: n, total_bytes, capacity
          integer(c_int) :: status
       end function
       ! ---- window forms: one text split across GPUs (one MPI rank / coarray image per GPU; see INTEGRATION.md 3) ----
@@ -320,6 +343,7 @@ module forgex_b200_m
    public :: fx_in, fx_match, fx_regex, fx_in_value, fx_match_value, fx_regex_sub, fx_is_valid_regex, fx_compile_from_dfa
    public :: fx_match_fixed_dev, fx_in_fixed_dev, fx_match_batch_dev, fx_in_batch_dev, fx_regex_batch_dev, fx_regex_count_batch_dev
    public :: fx_regex_buffer_work_bytes, fx_regex_buffer_dev, fx_regex_buffer_all_dev
+   public :: fx_regex_all_batch_work_bytes, fx_regex_all_batch_dev
    public :: fx_buffer_scan_dev, fx_buffer_scan_all_dev, fx_buffer_finish_dev
    public :: fx_statemap_window_dev, fx_statemap_combine, fx_statemap_back_dev
 
@@ -413,6 +437,19 @@ contains
       integer, intent(out) :: status
       status = fx_regex_count_batch(pat%handle, buf, offsets, int(size(counts), c_int64_t), counts)
    end subroutine regex_count_batch
+
+   ! every match of every string: string i's spans are from(rows(i-1)+1 : rows(i)), to(...) (rows(0:n), rows(0) = 0),
+   ! in the string's own coordinates; rows is always complete, at most min(size(from), size(to)) spans are stored
+   subroutine regex_all_batch(pat, buf, offsets, rows, from, to, status)
+      type(fx_pattern_t), intent(in) :: pat
+      character(len=*), intent(in) :: buf
+      integer(int64), intent(in) :: offsets(0:)
+      integer(int64), intent(out) :: rows(0:)
+      integer(int64), intent(inout) :: from(:), to(:)
+      integer, intent(out) :: status
+      status = fx_regex_all_batch(pat%handle, buf, offsets, int(size(rows) - 1, c_int64_t), rows, from, to, &
+                                  int(min(size(from), size(to)), c_int64_t))
+   end subroutine regex_all_batch
 
    ! every match of one buffer, in order; at most size(from) spans are stored, count may be larger
    subroutine regex_buffer_all(pat, buf, from, to, count, status)

@@ -202,11 +202,25 @@ int fx_regex_buffer_dev(fx_pattern* p, const uint8_t* d_buf, int64_t len, int64_
  * fx_regex_count_batch*: the number of matches per string of a ragged batch (d_counts[n]).
  * fx_regex_buffer_all*: one buffer; the first `capacity` spans in whole-buffer coordinates, *count (HOST memory in both
  * forms) = the number of matches (may exceed capacity).  The _dev form synchronises `stream` (per far match, or per
- * thousand near ones) and needs fx_regex_buffer_work_bytes(len) bytes of scratch. */
+ * thousand near ones) and needs fx_regex_buffer_work_bytes(len) bytes of scratch.
+ * fx_regex_all_batch*: every match of every string of a ragged batch, as CSR rows + flat spans.  rows[n + 1]: rows[0] = 0
+ * and rows[i + 1] - rows[i] = the number of matches of string i (so rows[1..n] is the inclusive prefix sum of what
+ * fx_regex_count_batch returns, and rows[n] is the total).  from[k], to[k] for k in [rows[i], rows[i + 1]) are string
+ * i's matches in order, 1-based inclusive in the STRING's own coordinates (as fx_regex_batch returns them).  Only
+ * indices k < capacity are written; rows is always complete, so a caller can read rows[n] and call again with room for
+ * every span.  Every match advances the rest by at least one byte, so rows[n] <= total_bytes: a capacity of
+ * total_bytes is always enough.  The _dev form is fully asynchronous (no host sync, nothing read back): the counts go
+ * to d_rows + 1, d_rows[0] = 0 (also for n = 0), d_rows[1..n] is scanned in place, then the span pass runs -- not at
+ * all for capacity 0, a cheap "rows only" call.  d_work: fx_regex_all_batch_work_bytes(n) bytes of device scratch,
+ * 8-byte aligned (8 bytes per block of the scan, one block per 1024 strings up to 1024 blocks: at most 8 KB; computed
+ * on the host).  Status codes are those of fx_regex_count_batch*. */
 int fx_regex_count_batch_dev(fx_pattern* p, const uint8_t* d_buf, const int64_t* d_offsets, int64_t n, int64_t total_bytes,
                              int64_t* d_counts, void* stream);
 int fx_regex_buffer_all_dev(fx_pattern* p, const uint8_t* d_buf, int64_t len, int64_t* d_from, int64_t* d_to, int64_t capacity,
                             int64_t* count, void* d_work, void* stream);
+int64_t fx_regex_all_batch_work_bytes(int64_t n);
+int fx_regex_all_batch_dev(fx_pattern* p, const uint8_t* d_buf, const int64_t* d_offsets, int64_t n, int64_t total_bytes,
+                           int64_t* d_rows, int64_t* d_from, int64_t* d_to, int64_t capacity, void* d_work, void* stream);
 
 /* Window forms of the buffer search, for a text that is split across GPUs.  A window is a contiguous piece of the
  * text held by this GPU: window byte 0 is text position `origin` (0-based).  fx_buffer_scan_dev tries the starts
@@ -270,6 +284,8 @@ int fx_regex_batch(fx_pattern* p, const uint8_t* buf, const int64_t* offsets, in
 int fx_regex_buffer(fx_pattern* p, const uint8_t* buf, int64_t len, int64_t* from, int64_t* to);
 int fx_regex_count_batch(fx_pattern* p, const uint8_t* buf, const int64_t* offsets, int64_t n, int64_t* counts);
 int fx_regex_buffer_all(fx_pattern* p, const uint8_t* buf, int64_t len, int64_t* from, int64_t* to, int64_t capacity, int64_t* count);
+int fx_regex_all_batch(fx_pattern* p, const uint8_t* buf, const int64_t* offsets, int64_t n, int64_t* rows, int64_t* from,
+                       int64_t* to, int64_t capacity);
 
 /* ---- one pattern, one text: the reference's public API, compiled per call like the reference does */
 int fx_in(const void* pattern, int64_t plen, const void* text, int64_t tlen, int* result);
